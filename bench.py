@@ -2,7 +2,7 @@
 """Benchmark of the MultiAgentEnv.step hot path (BASELINE.json metric: batched env-steps/s
 incl. power flow).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload = "C1"): the reference's IEEE-13 coordinated-buildings scenario
 (3 x building+PV+storage on load 675c, load factor 1.2, shared voltage penalty;
@@ -325,6 +325,34 @@ def _ncu_capture(workload, E):
     return res
 
 
+DUMP_MAX_BYTES = 64 * 10 ** 6
+
+
+def _dump_outputs(out_dir, batches):
+    """--dump-outputs: what the timed path handed its caller at the last timed step -- each batch's
+    observations [obs_dim, E], rewards [agents, E] (float64) and done flags [E] (float32) -- as
+    out_dir/<prefix>obs.npy, <prefix>reward.npy, <prefix>done.npy.  ``batches`` maps a file-name
+    prefix to an env.  Above DUMP_MAX_BYTES in all, every batch keeps the same share of its env
+    columns, drawn by a fixed seed; their indices go to <prefix>env_index.npy (float64)."""
+    import numpy as np
+    per_env = {p: 8 * env.obs_dim + 8 * len(env.agents) + 4 for p, env in batches.items()}
+    total = sum(per_env[p] * env.num_envs for p, env in batches.items())
+    budget = DUMP_MAX_BYTES - 4096                   # room for the .npy headers
+    share = 1.0 if total <= budget else \
+        budget / sum((per_env[p] + 8) * env.num_envs for p, env in batches.items())
+    os.makedirs(out_dir, exist_ok=True)
+    for prefix, env in batches.items():
+        arrays = {"obs": env.obs.cpu().numpy(), "reward": env.rew.cpu().numpy(),
+                  "done": env.done.cpu().numpy().astype(np.float32)}
+        if share < 1.0:
+            keep = max(1, int(env.num_envs * share))
+            cols = np.sort(np.random.default_rng(0).choice(env.num_envs, size=keep, replace=False))
+            arrays = {k: v[..., cols] for k, v in arrays.items()}
+            arrays["env_index"] = cols.astype(np.float64)
+        for name, arr in arrays.items():
+            np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), np.ascontiguousarray(arr))
+
+
 def _bind_to_gpu_numa(index):
     """Run this rank (and first-touch its pinned buffers) on the CPUs next to its GPU."""
     try:
@@ -356,9 +384,10 @@ def _component_bytes(env, workload, E, W, K):
     return alg, survey
 
 
-def measure(workload, E, K, W, dev, world=1, rank=0, headline=False, pdl=1):
+def measure(workload, E, K, W, dev, world=1, rank=0, headline=False, pdl=1, dump_dir=None):
     """One workload on this rank's GPU: K device-timed steps with a cold L2 before each, the
-    per-kernel durations of the same loop, and the rooflines they give."""
+    per-kernel durations of the same loop, and the rooflines they give.  With ``dump_dir``, rank 0
+    writes the outputs of the last timed step there (_dump_outputs)."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -427,6 +456,8 @@ def measure(workload, E, K, W, dev, world=1, rank=0, headline=False, pdl=1):
     wall = time.perf_counter() - wall0
     step_ms = [s.elapsed_time(e) for s, e in zip(starts, ends)]
     total_ms = float(sum(step_ms))
+    if dump_dir is not None and rank == 0:            # before the passes below overwrite them
+        _dump_outputs(dump_dir, {"": env})
     iters_mean = float(env.get_field(7).abs().double().mean()) if has_pf else 0.0
     if world > 1:
         t = torch.tensor([total_ms], device=dev, dtype=torch.float64)
@@ -584,7 +615,8 @@ def run_ours(args):
     E = ENVS_PER_GPU
     stream = torch.cuda.Stream(dev)                   # a non-default stream: pgw_step replays its graph
     torch.cuda.set_stream(stream)
-    m = measure(WORKLOAD, E, K, W, dev, world, rank, headline=True, pdl=args.pdl)
+    m = measure(WORKLOAD, E, K, W, dev, world, rank, headline=True, pdl=args.pdl,
+                dump_dir=args.dump_outputs)
     env, A, has_pf = m["env"], m["A"], m["has_pf"]
     barrier, one_step, begin_pass, soc = m["barrier"], m["one_step"], m["begin_pass"], m["soc"]
 
@@ -805,6 +837,8 @@ def run_mix(args):
         step_all(W + i, fence=starts[i])
         ends[i].record(main_stream)
     barrier()
+    if args.dump_outputs is not None and rank == 0:
+        _dump_outputs(args.dump_outputs, {f"{pt['wl']}_": pt["env"] for pt in parts})
     launches = sum(pt["env"].launch_count for pt in parts) - launches0
     sampler.stop_flag = True
     total_ms = float(sum(s_.elapsed_time(e_) for s_, e_ in zip(starts, ends)))
@@ -894,7 +928,14 @@ def main():
                     help="envs per GPU (default: 4096 for C1, 65536 for C2, 16384 for C3)")
     ap.add_argument("--pf-kernel", default=PF_KERNEL, choices=["fp64", "tc", "tc2"])
     ap.add_argument("--workload", default="c1", choices=["c1", "c2", "c3", "c4", "hs"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the observations, rewards and done flags of the last timed step as "
+                         "DIR/*.npy (rank 0's envs; a seeded sample of env columns above 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.envs is None and args.workload != "c4":
         args.envs = {"c1": 4096, "c2": 65536, "c3": 16384, "hs": 262144}[args.workload]
     ENVS_PER_GPU, PF_KERNEL, WORKLOAD, GRAPHS = args.envs, args.pf_kernel, args.workload, args.graphs
