@@ -152,7 +152,7 @@ struct pgw_env {
   // fused step kernel (step_fused.cu): eligible scenario, and PGW_OPT_FUSED (0 off, 1 auto: batches
   // of at most two 32-env tiles per SM, 2 always)
   bool fused_ok = false;
-  int fused_mode = 1, fused_tmem_cols = 0;
+  int fused_mode = 1;
   bool clip_init_soc = true;
   // device state
   double* sd = nullptr;
@@ -820,6 +820,16 @@ int pgw_create(const pgw_spec* spec, pgw_env** out) {
         t.f_kc = putf(&env->tc2c, sizeof(env->tc2c));
         t.f_kp = putf(&env->tc2p, sizeof(env->tc2p));
         t.f_aslot = putf(aslot.data(), aslot.size() * 4);
+        // Znb^T / xscale of the expansion slots in float32 ([k][slot], 16 ncc slots a row): the
+        // fused kernel's v = w - Znb i on the SIMT pipe, from the fixed point's scaled currents
+        const int nxs = NBP * ncc;
+        std::vector<float2> xz((size_t)NBP * nxs, make_float2(0.f, 0.f));
+        for (int k = 0; k < nb; ++k)
+          for (int sidx = 0; sidx < nx; ++sidx) {
+            const double2 z = ZN(xnode[sidx], k);
+            xz[(size_t)k * nxs + sidx] = make_float2((float)(z.x / xs), (float)(z.y / xs));
+          }
+        t.f_xz = putf(xz.data(), xz.size() * sizeof(float2));
         blob.resize((blob.size() + 15) / 16 * 16, 0);
         t.ftab_bytes = (int)(blob.size() - (size_t)t.off_ftab);
       }
@@ -828,18 +838,15 @@ int pgw_create(const pgw_spec* spec, pgw_env** out) {
       if (pgw::tc2_smem_bytes(probe) + 6 * 1024 <= 227 * 1024) {   // + the kernel's static arrays
         PGW_TRY(upload(&env->tc2_blob, blob.data(), blob.size())); env->own(env->tc2_blob);
         env->tc2.blob = env->tc2_blob;
-        // The fused step kernel serves feeders with <= 16 load branches whose Znb chunks stay
-        // resident, stock components on their straight-line paths, tables that fit shared memory.
-        bool ok = nch == 2 && t.resident && !env->has_house && !env->ev_per_env && !env->need_scratch &&
-                  32 * (1 + ncc) <= 512;
+        // The fused step kernel serves feeders with <= 16 load branches, stock components on their
+        // straight-line paths, tables that fit shared memory.
+        bool ok = nch == 2 && !env->has_house && !env->ev_per_env && !env->need_scratch;
         for (int c = 0; c < spec->num_components && ok; ++c) {
           const pgw_component& k = spec->components[c];
           ok = k.type >= PGW_STORAGE && k.type <= PGW_BUILDING &&
                (k.type != PGW_BUILDING || (k.flags & PGW_F_BUILDING_FAST));
         }
         if (ok) {
-          env->fused_tmem_cols = 32;
-          while (env->fused_tmem_cols < 32 * (1 + ncc)) env->fused_tmem_cols *= 2;
           pgw::FusedParams P{};
           P.c.blob_bytes = env->comp_blob_bytes; P.c.dstride = env->dstride; P.c.istride = env->istride;
           P.f.tc2 = t; P.C = env->C; P.act_dim = env->act_dim;
@@ -1022,7 +1029,7 @@ static pgw::FusedParams step_fused_params(pgw_env* env, const double* actions, d
   P.event = event;
   P.c = step_comp_params(env, actions, obs, rew, done, e_lo, e_hi, 1, 0);
   P.f = step_pf_params(env, rew, e_lo, e_hi, 1u, false);
-  P.C = env->C; P.act_dim = env->act_dim; P.sd_rows = env->sd_rows; P.e_lo = e_lo; P.e_hi = e_hi; P.tmem_cols = env->fused_tmem_cols;
+  P.C = env->C; P.act_dim = env->act_dim; P.sd_rows = env->sd_rows; P.e_lo = e_lo; P.e_hi = e_hi;
   P.tickets = tickets ? tickets : (unsigned int)fused_grid(e_hi - e_lo);
   P.stagger_cycles = stagger;
   return P;

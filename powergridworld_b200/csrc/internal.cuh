@@ -112,7 +112,9 @@ struct Tc2Params {
   // from shared memory -- warp-uniform broadcasts -- instead of the parameter constant bank, whose
   // 7 kB are cold in every SM's constant cache at every launch) and, per agent, the load branch
   // whose wye node is the agent's bus (-1: none).  pen_slot: the same for the penalty node.
-  int off_ftab, ftab_bytes, f_kc, f_kp, f_aslot, pen_slot;
+  // f_xz: Znb^T / xscale of the node-voltage expansion in float32, [16 branches][16 ncc slots]
+  // (f_xz[k * 16 ncc + s] = Znb[xnode[s]][k] / xscale, zero padded).
+  int off_ftab, ftab_bytes, f_kc, f_kp, f_aslot, f_xz, pen_slot;
   float xscale, descale1, descale2, tol;
 };
 
@@ -173,7 +175,6 @@ struct FusedParams {
   int act_dim;             // action rows per env
   int sd_rows;             // double state rows per env
   int e_lo, e_hi;
-  int tmem_cols;           // 32 x (1 + Znb chunks), rounded up to a power of two
   unsigned int tickets;    // CTAs of all launches of this step (the last one advances the clock)
   int stagger_cycles;      // CTA b delays the fetch of its first tile's actions by b x this many SM
                            // cycles (actions in host memory: requests served in tile order, so that

@@ -2,7 +2,7 @@
 // gridworld/multiagent_env.py:165-189 + the OpenDSS solve of distribution_system/opendss.py:134
 // + the reward hook of examples/marl/openai/train.py:51-88 for a tile of envs):
 //
-//   component steps  ->  nominal power of the load branches  ->  tcgen05 split-FP16 fixed point
+//   component steps  ->  nominal power of the load branches  ->  float32 fixed point
 //   ->  float64 polish  ->  node-voltage expansion  ->  bus voltages, penalty, rewards
 //
 // A CTA of 512 threads owns a tile of 32 envs end to end.  Thread (w, e): warp w, lane e = env
@@ -15,23 +15,22 @@
 //   observations and state, and leaves real power and reward in shared memory; the agents'
 //   sums (in component order, as the reference adds them) stay on chip -- no agent_p / reward
 //   round trip through HBM, no second launch, one clock read, one staging of the event row.
-// * Power flow: warp w owns load branch w.  The env tile sits on the MMA M dimension four
-//   times over (A row 32 q + e = env e for every TMEM lane quadrant q), so each warp reads
-//   the voltage drop of ITS branch from ITS quadrant with two one-column tcgen05.ld; the
-//   contraction D[128, 32] = A[128, 32] B^T (B = real-ified Zbb, FP16 hi/lo images prepared on
-//   the host, the same images powerflow_tc2.cu uses) is 6 tcgen05.mma.kind::f16 per iteration
-//   (x_lo B_hi + x_hi B_lo + x_hi B_hi, FP32 accumulation in TMEM).  Currents go through a
-//   small staging array ([k][env], conflict free) from which eight warps build the 16-byte
-//   rows of the canonical K-major A images; one CTA barrier and one mbarrier hand-off per
-//   iteration.  Per-env convergence: max |d drop| over the env's 16 branch threads through a
-//   shared-memory atomicMax; converged envs freeze their currents (their drop reproduces
-//   itself); every warp knows `all envs converged` from a vote over its own lanes.
-// * Polish: float64 sweeps u <- u0 - Zbb i(u) on the SIMT pipe, one branch per thread (Zbb row
-//   from the constant bank, the env's currents through shared memory), spread over 16 warps and
-//   -- with 32-env tiles -- over every SM of the GPU: ~0.4 us per sweep at 4096 envs instead of
-//   ~3 us in the 128-env tiles of powerflow_tc2.cu.
-// * Expansion v = w - Znb i for the nodes that are not a wye-load node: the same chain against
-//   the resident Znb chunk images into accumulators of their own, one node slot per thread.
+// * Power flow: warp w owns load branch w.  One iteration of u <- u0 - Zbb i(u) is: the current
+//   of my branch into a [k][env] float2 array (conflict free, double-buffered by iteration
+//   parity), one CTA barrier, then the new drop of my branch from the env's nb currents against
+//   the Zbb row (Zbb^T / xscale in shared memory, warp-uniform broadcasts), two FFMA chains on
+//   the FP32 pipe.  At 32 envs per tile a tensor-core contraction buys nothing: its latency was
+//   the hand-offs around the MMA (DESIGN.md section 4.3d).  Per-env convergence: max |d drop|
+//   over the env's 16 branch threads through a shared-memory atomicMax; converged envs freeze
+//   their currents (their drop reproduces itself); every warp knows `all envs converged` from a
+//   vote over its own lanes.
+// * Polish: the fixed point's iteration once more with correctly rounded currents, then float64
+//   sweeps u <- u0 - Zbb i(u) on the SIMT pipe, one branch per thread (the env's currents through
+//   shared memory), spread over 16 warps and -- with 32-env tiles -- over every SM of the GPU:
+//   ~0.4 us per sweep at 4096 envs instead of ~3 us in the 128-env tiles of powerflow_tc2.cu.
+// * Expansion v = w - Znb i for the nodes that are not a wye-load node: the same float32 row
+//   product against Znb^T / xscale from the fixed point's final currents, one node slot per
+//   thread and chunk of 16 slots.
 //
 // Compiled -fmad=false like components.cu (the component arithmetic must round like NumPy);
 // the power-flow code spells out its fused multiply-adds.
@@ -45,22 +44,9 @@ namespace pgw {
 constexpr int SF_ENVS = 32;                            // envs per tile = lanes of a warp
 constexpr int SF_WARPS = 16;
 constexpr int SF_THREADS = SF_ENVS * SF_WARPS;
-constexpr int SF_N = 32;                               // MMA N = K: 16 branches x (Re, Im)
-constexpr uint32_t SF_SBO = 512;                       // bytes between 8-row groups (K = 32 halves)
-constexpr uint32_t SF_PB = (SF_N / 8) * SF_SBO;        // one B image: 32 rows
-constexpr uint32_t SF_APB = 16 * SF_SBO;               // one A image: 128 rows
-
-__device__ __forceinline__ float sf_ld1(uint32_t taddr) {
-  uint32_t r;
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x1.b32 {%0}, [%1];" : "=r"(r) : "r"(taddr));
-  return __uint_as_float(r);
-}
-__device__ __forceinline__ void sf_wait_ld() {
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
 
 struct SfLayout {                                      // byte offsets into dynamic shared memory
-  uint32_t b, a, stage, tab, ftab, blob, drow, irow, i64, dmax, part, vn, cp, cr, act, total;
+  uint32_t tab, ftab, blob, drow, irow, i32, i64, dmax, part, vn, cp, cr, act, total;
 };
 
 __host__ __device__ inline SfLayout sf_layout(const FusedParams& P) {
@@ -71,16 +57,14 @@ __host__ __device__ inline SfLayout sf_layout(const FusedParams& P) {
     o += (bytes + 127u) & ~127u;
     return at;
   };
-  L.b = take((uint32_t)(1 + P.f.tc2.ncc) * 2u * SF_PB);
-  L.a = take(2u * SF_APB);
-  L.stage = take(2u * 32u * SF_ENVS * 2u);             // hi | lo: [32 k][32 envs] halves
   L.tab = take((uint32_t)P.f.tc2.tab_bytes);
   L.ftab = take((uint32_t)P.f.tc2.ftab_bytes);
   L.blob = take((uint32_t)P.c.blob_bytes);
   L.drow = take((uint32_t)P.c.dstride * 8u);
   L.irow = take((uint32_t)P.c.istride * 4u + 16u);
+  L.i32 = take(2u * 16u * SF_ENVS * 8u);               // fixed-point currents, [parity][k][env] float2
   L.i64 = take(16u * SF_ENVS * 16u);                   // currents of a polish sweep
-  L.dmax = take(2u * SF_ENVS * 4u);
+  L.dmax = take(3u * SF_ENVS * 4u);
   L.part = take(2u * 16u * SF_ENVS * 4u);              // per-branch min / max |v| partials
   L.vn = take(16u * SF_ENVS * 8u);                     // |v| of each branch's wye node (penalty, bus voltages)
   L.cp = take((uint32_t)P.C * SF_ENVS * 8u);           // component real power
@@ -111,8 +95,7 @@ template <bool ANY_M5>
 __global__ void __launch_bounds__(SF_THREADS, 1)
     step_fused_kernel(const __grid_constant__ FusedParams P) {
   extern __shared__ __align__(1024) unsigned char sf_smem[];
-  __shared__ __align__(8) uint64_t mbar_tab, mbar_ev, mbar_b, mbar_mma, mbar_a, mbar_act;
-  __shared__ uint32_t tmem_base_s;
+  __shared__ __align__(8) uint64_t mbar_tab, mbar_ev, mbar_act;
   const CompParams& pc = P.c;
   const PfParams& pf = P.f;
   const Tc2Params& t = pf.tc2;
@@ -122,9 +105,6 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   const int w = __shfl_sync(0xffffffffu, tid >> 5, 0);  // provably warp uniform
   const int E = pc.E;
 
-  unsigned char* sB = sf_smem + L.b;
-  unsigned char* sA = sf_smem + L.a;
-  __half* sStage = reinterpret_cast<__half*>(sf_smem + L.stage);   // [part][k][env]
   unsigned char* sT = sf_smem + L.tab;
   // per-branch constants of the load model and the float64 polish tables: shared memory, every
   // read a warp-uniform broadcast (as kernel parameters they were 7 kB of cold constant-cache lines)
@@ -132,11 +112,13 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   const Tc2Polish& kp = *reinterpret_cast<const Tc2Polish*>(sf_smem + L.ftab + t.f_kp);
   const int32_t* aslot = reinterpret_cast<const int32_t*>(sf_smem + L.ftab + t.f_aslot);
   const float2* z32 = kp.z32;                          // Zbb^T / xscale
+  const float2* xz = reinterpret_cast<const float2*>(sf_smem + L.ftab + t.f_xz);   // Znb^T / xscale, [k][slot]
   unsigned char* sBlob = sf_smem + L.blob;
   double* drow = reinterpret_cast<double*>(sf_smem + L.drow);
   int32_t* irow = reinterpret_cast<int32_t*>(sf_smem + L.irow);
+  float2* sI32 = reinterpret_cast<float2*>(sf_smem + L.i32);       // [2][16][env]
   double2* sI64 = reinterpret_cast<double2*>(sf_smem + L.i64);
-  int* sDmax = reinterpret_cast<int*>(sf_smem + L.dmax);           // [2][env] float bits
+  int* sDmax = reinterpret_cast<int*>(sf_smem + L.dmax);           // [3][env] float bits
   float* sVmn = reinterpret_cast<float*>(sf_smem + L.part);        // [16][env]
   float* sVmx = sVmn + 16 * SF_ENVS;
   double* sVn = reinterpret_cast<double*>(sf_smem + L.vn);         // [16][env]
@@ -144,7 +126,7 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   double* sCr = reinterpret_cast<double*>(sf_smem + L.cr);
   double* sAct = reinterpret_cast<double*>(sf_smem + L.act);
 
-  // ---- prologue: clock, staging of everything that is shared by the envs, TMEM
+  // ---- prologue: clock, staging of everything that is shared by the envs
   bool first_tile = true;
 #ifdef PGW_PHASE_TIMERS
   if (pf.phase_clk != nullptr && threadIdx.x == 0) pf.phase_clk[(size_t)(blockIdx.x + P.e_lo / SF_ENVS) * 16 + 12] = (long long)global_timer_ns();
@@ -221,16 +203,10 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   if (tid == 0) {
     mbar_init(&mbar_tab, 1);
     mbar_init(&mbar_ev, 1);
-    mbar_init(&mbar_b, 1);
-    mbar_init(&mbar_mma, 1);
-    mbar_init(&mbar_a, 8);                             // one arrival per repacking warp
     mbar_expect_tx(&mbar_tab, (uint32_t)t.tab_bytes + (uint32_t)t.ftab_bytes + (uint32_t)pc.blob_bytes);
     tma_bulk_g2s(sBlob, pc.blob, (uint32_t)pc.blob_bytes, &mbar_tab);
     tma_bulk_g2s(sT, t.blob + t.off_tab, (uint32_t)t.tab_bytes, &mbar_tab);
     tma_bulk_g2s(sf_smem + L.ftab, t.blob + t.off_ftab, (uint32_t)t.ftab_bytes, &mbar_tab);
-    const uint32_t img = (uint32_t)(1 + t.ncc) * 2u * SF_PB;
-    mbar_expect_tx(&mbar_b, img);
-    tma_bulk_g2s(sB, t.blob, img, &mbar_b);            // Zbb images, then the Znb chunks
     // last: the event row's address waits for the device clock
     const uint32_t dbytes = (uint32_t)pc.dstride * 8u, ibytes = (uint32_t)pc.istride * 4u;
     mbar_expect_tx(&mbar_ev, dbytes + ibytes);
@@ -238,21 +214,7 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
     if (ibytes) tma_bulk_g2s(irow, pc.itab + (size_t)event * pc.istride, ibytes, &mbar_ev);
     if (!host_event) my_ticket = clock_take_ticket(pc.ticket, clk);
   }
-  if (w == 0) {                                        // one warp owns TMEM alloc / free
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                     smem_u32(&tmem_base_s)),
-                 "r"((uint32_t)P.tmem_cols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  // A rows and the staging array start from zero: the padded branches never write, and the MMA
-  // reads all 128 rows from its first use on
-  for (int i = tid; i < (int)(2u * SF_APB + 2u * 32u * SF_ENVS * 2u) / 16; i += SF_THREADS)
-    reinterpret_cast<uint4*>(sA)[i] = make_uint4(0u, 0u, 0u, 0u);   // sA and sStage are adjacent
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem = tmem_base_s;
+  __syncthreads();                                     // barriers initialised
   SF_STAMP(1);
   mbar_wait(&mbar_tab, 0);
   SF_STAMP(2);
@@ -290,82 +252,24 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   io.irow = irow;
 
   const int b = w;                                     // my load branch
-  const int bc = b >> 3, bj = b & 7;
-  const int kre = 16 * bc + bj, kim = kre + 8;         // K / N position of Re and Im of branch b
-  const uint32_t t_lane = tmem + ((uint32_t)((w & 3) * 32) << 16);
-  const uint32_t idesc = t2_idesc_f16(SF_N);
-  const uint32_t sA_u = smem_u32(sA), sB_u = smem_u32(sB);
-  const float xs = t.xscale, ds1 = t.descale1, ds2 = t.descale2;
+  const float xs = t.xscale, ds1 = t.descale1;
+  const float rds1 = 1.f / ds1;                        // a power of two: the rescaling is exact
   const float tol_s = t.tol / ds1;
   const float4 cst = t2_cst(kc, b);
   const float2 gh = ANY_M5 ? t2_gh(kc, b) : make_float2(1.f, 0.f);
-  uint32_t mma_phase = 0, a_phase = 0;
 
-  // One accumulation chain D = A_lo B_hi + A_hi B_lo + A_hi B_hi (small terms first) into the
-  // accumulator at column d_col against the image pair at byte offset b_off.
-  auto chain = [&](uint32_t d_col, uint32_t b_off) {
-    const uint64_t a_hi = t2_smem_desc(sA_u, SF_SBO), a_lo = t2_smem_desc(sA_u + SF_APB, SF_SBO);
-    const uint64_t b_hi = t2_smem_desc(sB_u + b_off, SF_SBO), b_lo = t2_smem_desc(sB_u + b_off + SF_PB, SF_SBO);
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk)
-      t2_umma_f16(tmem + d_col, a_lo + 16u * kk, b_hi + 16u * kk, idesc, kk > 0 ? 1u : 0u);
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk) t2_umma_f16(tmem + d_col, a_hi + 16u * kk, b_lo + 16u * kk, idesc, 1u);
-#pragma unroll
-    for (int kk = 0; kk < 2; ++kk) t2_umma_f16(tmem + d_col, a_hi + 16u * kk, b_hi + 16u * kk, idesc, 1u);
-  };
-  // Currents of my branch into the staging array: [part][k][env] halves.
-  auto stage_current = [&](float x, float y) {
-    const uint32_t hi = t2_pack(x, y);
-    const float2 back = __half22float2(*reinterpret_cast<const __half2*>(&hi));
-    const uint32_t lo = t2_pack(x - back.x, y - back.y);
-    const __half2 h2 = *reinterpret_cast<const __half2*>(&hi), l2 = *reinterpret_cast<const __half2*>(&lo);
-    sStage[kre * SF_ENVS + lane] = __low2half(h2);
-    sStage[kim * SF_ENVS + lane] = __high2half(h2);
-    sStage[(32 + kre) * SF_ENVS + lane] = __low2half(l2);
-    sStage[(32 + kim) * SF_ENVS + lane] = __high2half(l2);
-  };
-  // Warps 0..7: one 16-byte chunk (8 K positions of one part) of every env's A row, written to
-  // the four replicas of the row (one per TMEM lane quadrant); then the hand-off to the issuer.
-  auto repack = [&]() {
-    if (w < 8) {
-      const int part = w >> 2, ch = w & 3;
-      const __half* src = sStage + (size_t)(part * 32 + 8 * ch) * SF_ENVS + lane;
-      uint32_t v[4];
-#pragma unroll
-      for (int q = 0; q < 4; ++q) {
-        const __half2 h = __halves2half2(src[(2 * q) * SF_ENVS], src[(2 * q + 1) * SF_ENVS]);
-        v[q] = *reinterpret_cast<const uint32_t*>(&h);
-      }
-      const uint4 val = make_uint4(v[0], v[1], v[2], v[3]);
-      unsigned char* dst = sA + (size_t)part * SF_APB + (size_t)(lane >> 3) * SF_SBO + (size_t)ch * 128 +
-                           (size_t)(lane & 7) * 16;
-#pragma unroll
-      for (int q = 0; q < 4; ++q) *reinterpret_cast<uint4*>(dst + (size_t)(4 * q) * SF_SBO) = val;
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&mbar_a);
+  // acc - sum_k z[k zs] i_k over the nb currents of my env (cur: [k][env], scaled by xscale like
+  // t2_current's; z: a column of Zbb^T or Znb^T over xscale, warp-uniform broadcasts): two FFMA
+  // chains on the FP32 pipe, summed at the end.
+  auto zdot = [&](float2 acc, const float2* z, int zs, const float2* cur) {
+    float2 a1 = make_float2(0.f, 0.f);
+#pragma unroll 2
+    for (int jj = 0; jj + 1 < pf.nb; jj += 2) {
+      t2_cmac_sub32(acc, z[jj * zs], cur[jj * SF_ENVS + lane]);
+      t2_cmac_sub32(a1, z[(jj + 1) * zs], cur[(jj + 1) * SF_ENVS + lane]);
     }
-  };
-  // Warp 15: wait for the repacked A, then issue either the next chain of the fixed point or --
-  // once every env of the tile has converged -- the expansion chains.
-  auto issue = [&](bool expansion) {
-    if (w == SF_WARPS - 1) {
-      if (t2_elect_one()) {
-        mbar_wait(&mbar_a, a_phase);
-        if (first_tile) mbar_wait(&mbar_b, 0);         // operand images have landed
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        if (!expansion) {
-          chain(0u, 0u);
-          t2_commit(&mbar_mma);
-        } else if (t.ncc > 0) {
-          for (int cc = 0; cc < t.ncc; ++cc) chain((uint32_t)((1 + cc) * SF_N), (uint32_t)(1 + cc) * 2u * SF_PB);
-          t2_commit(&mbar_mma);
-        }
-      }
-      __syncwarp();
-    }
-    a_phase ^= 1u;
+    if (pf.nb & 1) t2_cmac_sub32(acc, z[(pf.nb - 1) * zs], cur[(pf.nb - 1) * SF_ENVS + lane]);
+    return make_float2(acc.x + a1.x, acc.y + a1.y);
   };
 
   uint32_t act_phase = 0;
@@ -379,7 +283,7 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
     if (pf.warm_start && b < pf.nb) up = pf.u_state[(size_t)b * E + e];
     double er0 = 0.0;
     if (w < pc.A) er0 = pf.ep_ret[(size_t)w * E + e];
-    if (w < 2) sDmax[w * SF_ENVS + lane] = 0;
+    if (w < 3) sDmax[w * SF_ENVS + lane] = 0;
 
     if (first_tile) mbar_wait(&mbar_ev, 0);            // event row has landed
     if (tile_in_smem(tile)) {                          // CTA uniform
@@ -435,7 +339,7 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
     //      (multiagent_env.py:171-181: summed per load name in agent order; opendss.py:128)
     float sr = 0.f, si = 0.f;
     double2 s64 = make_double2(0.0, 0.0);
-    float2 dprev = make_float2(0.f, 0.f);
+    float2 dprev = make_float2(0.f, 0.f), cur = make_float2(0.f, 0.f);
     if (b < pf.nb) {
       const int l = bload[b];
       double ctl = 0.0;
@@ -451,84 +355,69 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
       si = (float)kvar * sh;
       s64 = make_double2(kw * kp.share[b], kvar * kp.share[b]);
       dprev = make_float2(((float)up.x - cst.x) * (1.f / ds1), ((float)up.y - cst.y) * (1.f / ds1));
-      float x, y;
-      t2_current<ANY_M5>(cst, gh, dprev.x, dprev.y, ds1, sr, si, x, y);
-      stage_current(x, y);
+      t2_current<ANY_M5>(cst, gh, dprev.x, dprev.y, ds1, sr, si, cur.x, cur.y);
+      sI32[b * SF_ENVS + lane] = cur;
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    repack();
-    issue(false);
     SF_STAMP(6);
 
-    // ---- fixed point
+    // ---- fixed point: iteration `it` reads the currents of parity (it - 1) & 1 and writes those
+    //      of parity it & 1 (one barrier per iteration); the convergence maxima rotate over three
+    //      slots, so that warp 0 can clear the next one before the barrier: every thread has read
+    //      it (two iterations ago) before it arrived at the previous barrier
     int it = 0, my_it = 0;
     bool conv = !valid, conv_ok = true;
     while (true) {
-      mbar_wait(&mbar_mma, mma_phase);
-      mma_phase ^= 1u;
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
       ++it;
-      float2 dn = make_float2(0.f, 0.f);
-      if (b < pf.nb) {                                 // warp uniform: tcgen05.ld is collective
-        dn.x = sf_ld1(t_lane + (uint32_t)kre);
-        dn.y = sf_ld1(t_lane + (uint32_t)kim);
-        sf_wait_ld();
+      const int slot = it % 3;
+      if (w == 0) sDmax[((it + 1) % 3) * SF_ENVS + lane] = 0;
+      if (b < pf.nb) {
+        const float2 d = zdot(make_float2(0.f, 0.f), z32 + b, 16, sI32 + ((it - 1) & 1) * 16 * SF_ENVS);
+        const float2 dn = make_float2(d.x * rds1, d.y * rds1);
         const float dd = fmaxf(fabsf(dn.x - dprev.x), fabsf(dn.y - dprev.y));
-        atomicMax(&sDmax[(it & 1) * SF_ENVS + lane], __float_as_int(dd));
-        if (!conv) {                                   // converged envs keep their currents
-          float x, y;
-          t2_current<ANY_M5>(cst, gh, dn.x, dn.y, ds1, sr, si, x, y);
-          stage_current(x, y);
-        }
+        atomicMax(&sDmax[slot * SF_ENVS + lane], __float_as_int(dd));
+        if (!conv) t2_current<ANY_M5>(cst, gh, dn.x, dn.y, ds1, sr, si, cur.x, cur.y);   // converged envs keep theirs
+        sI32[((it & 1) * 16 + b) * SF_ENVS + lane] = cur;
         dprev = dn;
       }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
       __syncthreads();
       if (!conv) {
-        const float d = __int_as_float(sDmax[(it & 1) * SF_ENVS + lane]);
+        const float d = __int_as_float(sDmax[slot * SF_ENVS + lane]);
         conv_ok = d < tol_s;
         conv = conv_ok || it >= pf.max_iter;
         my_it = it;
       }
-      const bool all_done = __all_sync(0xffffffffu, conv ? 1 : 0) != 0;
-      if (w == 0) sDmax[((it + 1) & 1) * SF_ENVS + lane] = 0;   // before my repack arrival
-      repack();
-      issue(all_done);
-      if (all_done) break;
+      if (__all_sync(0xffffffffu, conv ? 1 : 0) != 0) break;
     }
 
     SF_STAMP(7);
     [[maybe_unused]] const int it_stamp = it;
-    // ---- float64 polish of my branch voltage (the expansion chains run meanwhile)
+    const float2* i_fin = sI32 + (it & 1) * 16 * SF_ENVS;   // the fixed point's final currents
+    // ---- float64 polish of my branch voltage
     const bool polish = t.polish > 0 && pf.reward_hook;
     double2 u64 = make_double2(kp.u0[b].x + (double)dprev.x * (double)ds1,
                                kp.u0[b].y + (double)dprev.y * (double)ds1);
     const bool my_row = ((kp.rows >> b) & 1u) != 0u;
     if (polish) {
       const int sweeps = t.polish + ((kp.rows != 0u || t.polish_row >= 0) ? 1 : 0);
-      // Sweep 0 in float32.  A full sweep only has to take every branch voltage from the fixed
+      // Sweep 0 in float32: the fixed point's iteration once more, from its last drop, with
+      // correctly rounded reciprocals in the currents, into the other parity's array (free again:
+      // its last reader passed the loop's last barrier).  A full sweep only has to take every branch voltage from the fixed
       // point's ~1e-7 p.u. to ~1e-8: it feeds the currents of the next sweep, whose rows the rewards
       // read in float64, and a sweep contracts the error by more than 10x.  Float32 currents are
       // half the shared-memory traffic of the float64 sweep (every thread reads all currents of
       // its env: 14 warps x 14 x 512 B was the sweep's bound) and the FMAs run on the FP32 pipe.
       {
-        float2* sI32 = reinterpret_cast<float2*>(sI64);
+        float2* i_pre = sI32 + ((it + 1) & 1) * 16 * SF_ENVS;
         if (b < pf.nb) {
           float x, y;
           t2_current32<ANY_M5>(cst, gh, dprev.x, dprev.y, ds1, sr, si, x, y);
-          sI32[b * SF_ENVS + lane] = make_float2(x, y);
+          i_pre[b * SF_ENVS + lane] = make_float2(x, y);
         }
         __syncthreads();
         if (b < pf.nb) {
-          float2 a0 = make_float2(0.f, 0.f), a1 = make_float2(0.f, 0.f);
-#pragma unroll 2
-          for (int jj = 0; jj + 1 < pf.nb; jj += 2) {
-            t2_cmac_sub32(a0, z32[jj * 16 + b], sI32[jj * SF_ENVS + lane]);
-            t2_cmac_sub32(a1, z32[(jj + 1) * 16 + b], sI32[(jj + 1) * SF_ENVS + lane]);
-          }
-          if (pf.nb & 1) t2_cmac_sub32(a0, z32[(pf.nb - 1) * 16 + b], sI32[(pf.nb - 1) * SF_ENVS + lane]);
-          u64 = make_double2(kp.u0[b].x + (double)(a0.x + a1.x), kp.u0[b].y + (double)(a0.y + a1.y));
+          const float2 d = zdot(make_float2(0.f, 0.f), z32 + b, 16, i_pre);
+          u64 = make_double2(kp.u0[b].x + (double)d.x, kp.u0[b].y + (double)d.y);
           if (t.polish == 1 && valid) pf.u_state[(size_t)b * E + e] = u64;
         }
       }
@@ -572,32 +461,25 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
         if (valid) pf.vmag[(size_t)n * E + e] = mag;
       }
     }
-    if (t.ncc > 0) {
-      mbar_wait(&mbar_mma, mma_phase);
-      mma_phase ^= 1u;
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      for (int cc = 0; cc < t.ncc; ++cc) {
-        const int slot = 16 * cc + b;                  // warp uniform
-        if (slot < t.nx) {
-          const float vr0 = sf_ld1(t_lane + (uint32_t)((1 + cc) * SF_N + kre));
-          const float vi0 = sf_ld1(t_lane + (uint32_t)((1 + cc) * SF_N + kim));
-          sf_wait_ld();
-          const int n = xnode[slot];
-          if (n >= 0) {
-            const float2 wv = wx[slot];
-            const float vr = fmaf(vr0, ds2, wv.x), vi = fmaf(vi0, ds2, wv.y);
-            const float m2 = fmaf(vr, vr, vi * vi);
-            const float mag = m2 * t2_rsqrt(fmaxf(m2, 1e-30f));
-            vmn = fminf(vmn, mag);
-            vmx = fmaxf(vmx, mag);
-            if (valid) pf.vmag[(size_t)n * E + e] = (double)mag;
-          }
+    for (int cc = 0; cc < t.ncc; ++cc) {
+      const int slot = 16 * cc + b;                    // warp uniform
+      if (slot < t.nx) {
+        const int n = xnode[slot];
+        if (n >= 0) {
+          // - Znb i summed from zero (terms of the size of a drop), then w added once
+          const float2 dv = zdot(make_float2(0.f, 0.f), xz + slot, 16 * t.ncc, i_fin);
+          const float2 wv = wx[slot];
+          const float vr = wv.x + dv.x, vi = wv.y + dv.y;
+          const float m2 = fmaf(vr, vr, vi * vi);
+          const float mag = m2 * t2_rsqrt(fmaxf(m2, 1e-30f));
+          vmn = fminf(vmn, mag);
+          vmx = fmaxf(vmx, mag);
+          if (valid) pf.vmag[(size_t)n * E + e] = (double)mag;
         }
       }
     }
     sVmn[w * SF_ENVS + lane] = vmn;
     sVmx[w * SF_ENVS + lane] = vmx;
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();                                   // magnitudes (global) and partials visible
     SF_STAMP(9);
 
@@ -665,11 +547,6 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
     first_tile = false;
   }
 
-  __syncthreads();
-  if (w == 0)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem),
-                 "r"((uint32_t)P.tmem_cols)
-                 : "memory");
   if (tid == 0) {
     if (!host_event) clock_advance_if_last(my_ticket, pc.ticket, pc.clock, clk, P.tickets);
     else if (blockIdx.x == 0) *pc.clock = event;       // nobody reads it in this mode: any CTA may publish

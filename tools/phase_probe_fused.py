@@ -15,13 +15,16 @@ from powergridworld_b200 import _native as N  # noqa: E402
 
 SECOND = os.environ.get("PGW_PROBE_SECOND", "0") == "1"      # stamps of each CTA's second tile (build with
 #                                                               -DPGW_STAMP_SECOND_TILE, run with PGW_FUSED_GRID=64)
-N.LIB_PATH = os.path.join(ROOT, "tools", "_build", "libpgw_b200_phases2.so" if SECOND else "libpgw_b200_phases.so")
+# PGW_B200_LIB: another instrumented build (e.g. a parent commit's, for an A/B of the phases)
+N.LIB_PATH = os.environ.get("PGW_B200_LIB") or os.path.join(
+    ROOT, "tools", "_build", "libpgw_b200_phases2.so" if SECOND else "libpgw_b200_phases.so")
 from powergridworld_b200.scenarios import bench as SB  # noqa: E402
 
-PHASES = ["clock read + barrier init + TMA issue + TMEM alloc + zero A", "wait tables / component blob",
+PHASES = ["clock read + barrier init + TMA issue", "wait tables / component blob",
           "wait event row", "component steps (this thread's)", "barrier after the components",
-          "agent sums + nominal power + first currents + repack + issue", "fixed-point loop",
-          "float64 polish", "expansion + node magnitudes + barrier", "penalty, rewards, bus voltages"]
+          "agent sums + nominal power + first currents + barrier", "fixed-point loop",
+          "float32 pre-sweep + float64 polish", "expansion + node magnitudes + barrier",
+          "penalty, rewards, bus voltages"]
 
 
 def main():

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """How close the benchmarked solver's rewards come to the parity bound over whole episodes: fused step
-kernel (tcgen05 fixed point + float64 polish) against the FP64 SIMT solver, 4096 envs x 2 full episodes of
+kernel (float32 fixed point + float64 polish) against the FP64 SIMT solver, 4096 envs x 2 full episodes of
 random actions; prints the worst |error| / (2e-5 + 1e-5 |reward|) (must stay below 1) and the worst
 absolute error."""
 import json
@@ -19,7 +19,7 @@ st = torch.cuda.Stream()
 torch.cuda.set_stream(st)
 a = SB.c1_env(num_envs=E, pf_kernel="tc2")          # fused kernel (automatic at this size)
 b = SB.c1_env(num_envs=E, pf_kernel="fp64")
-if os.environ.get("PGW_TOL_NANO"):                   # convergence threshold of the tcgen05 loop, 1e-9 p.u. units
+if os.environ.get("PGW_TOL_NANO"):                   # convergence threshold of the fixed-point loop, 1e-9 p.u. units
     a.set_option(N.OPT_PF_TC_TOL_NANO, int(os.environ["PGW_TOL_NANO"]))
 gen = torch.Generator(device="cuda")
 gen.manual_seed(7)
