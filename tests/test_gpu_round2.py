@@ -189,13 +189,15 @@ def test_one_step_graph_serves_fresh_action_tensors(fused):
     assert 1e6 * host_s / T < 60.0
 
 
+@pytest.mark.parametrize("E", [2048 + 96, 7000])
 @pytest.mark.parametrize("fused", [0, 1])
-def test_host_step_zero_copy_staged_and_chunked_agree(fused):
+def test_host_step_zero_copy_staged_and_chunked_agree(fused, E):
     """pgw_step_host on page-locked buffers read / written in place, the same call staged through
     device buffers (one chunk and four pipelined chunks), a chain of zero-copy chunks, pageable
-    buffers (always staged) and the device-buffer path: identical results, bit for bit."""
+    buffers (always staged) and the device-buffer path: identical results, bit for bit.  E = 7000:
+    219 tiles of the fused kernel, so that CTAs of the one-chunk calls run two tiles."""
     torch = _torch()
-    E, T = 2048 + 96, 10
+    T = 10
     rng = np.random.default_rng(9)
     soc = rng.uniform(10, 40, size=(3, E))
     acts = rng.uniform(-1, 1, size=(T, 24, E))
@@ -370,27 +372,29 @@ def test_rllib_base_env_adapter_steps_a_batch_like_independent_envs():
 def test_event_index_and_device_clock_modes_interleave():
     """The fused step reads its event row through the host-supplied index when the graph's node
     parameters are rewritten for new caller buffers, and through the device clock when the same buffers
-    come again: any interleaving of the two gives the trajectory of a run on one buffer."""
+    come again: any interleaving of the two gives the trajectory of a run on one buffer.  At 300 envs
+    and at 7000, where CTAs run two tiles, of which only the first waits for the event row."""
     torch = _torch()
-    E, T = 300, 14
-    rng = np.random.default_rng(12)
-    soc = rng.uniform(10, 40, size=(3, E))
-    acts = rng.uniform(-1, 1, size=(T, 24, E))
-    a_env, b_env = (SB.c1_env(num_envs=E, pf_kernel="tc2") for _ in range(2))
-    st = torch.cuda.Stream()
-    with torch.cuda.stream(st):
-        a_env.reset_batch(soc), b_env.reset_batch(soc)
-        bufs = [torch.empty((24, E), dtype=torch.float64, device="cuda") for _ in range(3)]
-        pattern = [0, 1, 1, 1, 0, 0, 2, 1, 1, 2, 2, 2, 0, 1]          # which buffer each step uses
-        one = torch.empty((24, E), dtype=torch.float64, device="cuda")
-        for t in range(T):
-            x = torch.as_tensor(acts[t]).cuda()
-            bufs[pattern[t]].copy_(x)
-            one.copy_(x)
-            oa, ra, _, _ = a_env.step_batch(bufs[pattern[t]])
-            ob, rb, _, _ = b_env.step_batch(one)
-            assert torch.equal(oa, ob) and torch.equal(ra, rb), t
-        assert a_env._lib.pgw_graph_captures(a_env._h) == 1
-        assert a_env.episode_step == b_env.episode_step == T
-        assert torch.equal(a_env.get_field(N.FIELD_EP_RETURN), b_env.get_field(N.FIELD_EP_RETURN))
-    st.synchronize()
+    T = 14
+    for E in (300, 7000):
+        rng = np.random.default_rng(12)
+        soc = rng.uniform(10, 40, size=(3, E))
+        acts = rng.uniform(-1, 1, size=(T, 24, E))
+        a_env, b_env = (SB.c1_env(num_envs=E, pf_kernel="tc2") for _ in range(2))
+        st = torch.cuda.Stream()
+        with torch.cuda.stream(st):
+            a_env.reset_batch(soc), b_env.reset_batch(soc)
+            bufs = [torch.empty((24, E), dtype=torch.float64, device="cuda") for _ in range(3)]
+            pattern = [0, 1, 1, 1, 0, 0, 2, 1, 1, 2, 2, 2, 0, 1]          # which buffer each step uses
+            one = torch.empty((24, E), dtype=torch.float64, device="cuda")
+            for t in range(T):
+                x = torch.as_tensor(acts[t]).cuda()
+                bufs[pattern[t]].copy_(x)
+                one.copy_(x)
+                oa, ra, _, _ = a_env.step_batch(bufs[pattern[t]])
+                ob, rb, _, _ = b_env.step_batch(one)
+                assert torch.equal(oa, ob) and torch.equal(ra, rb), (E, t)
+            assert a_env._lib.pgw_graph_captures(a_env._h) == 1
+            assert a_env.episode_step == b_env.episode_step == T
+            assert torch.equal(a_env.get_field(N.FIELD_EP_RETURN), b_env.get_field(N.FIELD_EP_RETURN)), E
+        st.synchronize()

@@ -2,11 +2,14 @@
 point u <- u0 - Zbb i(u) with one branch per thread, currents scaled by xscale, the drop as two
 FFMA chains against Zbb^T / xscale, per-env convergence on max |d drop| with frozen currents,
 the float32 pre-sweep of the polish, and the expansion v = w - Znb i against Znb^T / xscale.
-Checks the accuracy claims of DESIGN.md 4.3d on the IEEE-13 feeder against a float64 solve."""
+Checks the accuracy claims of DESIGN.md 4.3d against a float64 solve, on the shipped IEEE-13 feeder
+and on the variants of the published one in tests/pf_reference.py (model-2/5 loads, 14, 15 and 16
+load branches)."""
 import numpy as np
 import pytest
 
 from powergridworld_b200.distribution_system.feeder import compile_feeder
+from tests.pf_reference import FEEDERS, band, feeder_file, solve64
 
 XS = 2048.0
 F32 = np.float32
@@ -17,20 +20,9 @@ def _fma(a, b, c):
     return (a.astype(np.float64) * b.astype(np.float64) + c.astype(np.float64)).astype(F32)
 
 
-@pytest.fixture(scope="module")
-def feeder():
-    return compile_feeder("ieee_13_dss/IEEE13Nodeckt.dss")
-
-
-def _band(f):
-    """clamp band of |u|^2 and the load characteristic per branch: k = 1 / clamp (models 1, 2),
-    1 / sqrt(clamp) with an open band (model 5)."""
-    m = np.asarray(f.branch_model)
-    lo = np.where(m == 2, 1.0, f.branch_vmin ** 2)
-    hi = np.where(m == 2, 1.0, f.branch_vmax ** 2)
-    lo = np.where(m == 5, 1e-30, lo)
-    hi = np.where(m == 5, 3e38, hi)
-    return lo, hi, m == 5
+@pytest.fixture(scope="module", params=FEEDERS)
+def feeder(request, tmp_path_factory):
+    return compile_feeder(feeder_file(request.param, tmp_path_factory.mktemp("feeder")))
 
 
 def _powers(f, load_scale):
@@ -38,25 +30,14 @@ def _powers(f, load_scale):
 
 
 def _solve64(f, load_scale):
-    """float64 fixed point to 1e-14: branch voltages and currents (p.u.)."""
-    lo, hi, m5 = _band(f)
-    s = _powers(f, load_scale) * f.branch_share * 1e-3
-    u = f.u0.copy()
-    for _ in range(200):
-        c = np.clip(np.abs(u) ** 2, lo, hi)
-        i = np.conj(s) * u / np.where(m5, np.sqrt(c), c)
-        un = f.u0 - f.zbb @ i
-        done = np.abs(un - u).max() < 1e-14
-        u = un
-        if done:
-            break
-    c = np.clip(np.abs(u) ** 2, lo, hi)
-    return u, np.conj(s) * u / np.where(m5, np.sqrt(c), c)
+    """float64 fixed point: branch voltages and currents (p.u.)."""
+    u, i, _ = solve64(f, _powers(f, load_scale) * f.branch_share * 1e-3)
+    return u[:, 0], i[:, 0]
 
 
 def _current32(f, d_re, d_im, sr, si):
     """t2_current32 on every branch: scaled currents of the drop (d_re, d_im) in float32."""
-    lo, hi, m5 = _band(f)
+    lo, hi, m5 = band(f)
     ur = (f.u0.real.astype(F32) + d_re).astype(F32)
     ui = (f.u0.imag.astype(F32) + d_im).astype(F32)
     m2 = _fma(ur, ur, (ui * ui).astype(F32))
