@@ -1,5 +1,6 @@
-"""Float64 reference of the power flow of one env step, and the IEEE-13 feeder variants that the
-fused-step tests run on.
+"""Float64 reference of the power flow of one env step, and the feeder variants that the
+power-flow kernel tests run on: IEEE-13 variants for the fused step, truncations and an extension
+of the packaged 123-bus-class feeder for the tc2 and FP64 kernels.
 
 ``solve64`` is the Z-bus fixed point u <- u0 - Zbb i(u) over a batch of envs with the load
 characteristic of the device tables (models 1 and 2 clamp |u|^2 to their band, model 5 draws a
@@ -46,6 +47,66 @@ def feeder_file(fid, directory):
     with open(path, "w") as fh:
         fh.writelines(out)
     return path
+
+
+SYNTHETIC123 = os.path.join(os.path.dirname(os.path.dirname(GOLD)), "powergridworld_b200", "data",
+                            "feeders", "synthetic123.dss")
+# loads copied (same bus, same kW / kvar) under a new name and a new model for the x100 variant:
+# 100 load branches, beyond tc2's 88 -> pf_fixed_point_kernel<32, 4, false> (nbp = 128)
+EXTRA_LOADS = (("37a", 1), ("58a", 2), ("56b", 5), ("18a", 1), ("33b", 2), ("111c", 5), ("4a", 1),
+               ("34a", 2), ("101a", 5), ("32b", 1), ("72a", 2), ("42a", 5), ("30b", 1), ("118a", 2),
+               ("117b", 5))
+
+
+def synthetic_feeder(directory, n_loads=85, extra=False):
+    """The packaged 123-bus-class feeder (85 single-phase wye loads) with only its first
+    ``n_loads`` loads, or (``extra``) with the loads of EXTRA_LOADS added as ``x<i>m<model>``."""
+    out, seen = [], 0
+    with open(SYNTHETIC123) as fh:
+        for line in fh:
+            if line.startswith("New Load."):
+                seen += 1
+                if seen > n_loads:
+                    continue
+                name = line.split()[1][5:]
+                for i, (src, model) in enumerate(EXTRA_LOADS if extra else ()):
+                    if src == name:
+                        out.append(line.replace(f"Load.{name} ", f"Load.x{i}m{model} ", 1)
+                                   .replace("Model=1", f"Model={model}"))
+            out.append(line)
+    path = os.path.join(str(directory), f"synthetic_{'x100' if extra else n_loads}.dss")
+    with open(path, "w") as fh:
+        fh.writelines(out)
+    return path
+
+
+def synthetic_config(ns, path, load_factor=0.9, hook_agents=0):
+    """Scenario on a synthetic123-class feeder.  ``hook_agents`` = 0: storage and PV agents spread
+    so that every rule of the branch powers and bus voltages is used -- three on the model-1 load
+    37a (summed in agent order; the third bus voltage goes past the two per-branch slots), two on
+    58a, one each on the model-5 load 5b and the model-2 load 20c (power ignored, bus voltage read),
+    one on the bus 10a that carries no load, one on 7b (a load of the full feeder only) and one on
+    4a.  ``hook_agents`` = n: n storage agents, all on 37a (the shared-penalty bus)."""
+    import pandas as pd
+    store = lambda kw: {"max_power": kw, "storage_range": (3., 80.)}
+    if hook_agents:
+        agents = [{"name": f"s{i}", "bus": "37a", "cls": ns.EnergyStorageEnv, "config": store(10. + i)}
+                  for i in range(hook_agents)]
+    else:
+        pv = lambda scale: {"profile_csv": "pv_profile.csv", "scaling_factor": scale}
+        roster = [("37a", ns.EnergyStorageEnv, store(60.)), ("37a", ns.PVEnv, pv(150.)),
+                  ("37a", ns.EnergyStorageEnv, store(25.)), ("58a", ns.EnergyStorageEnv, store(40.)),
+                  ("58a", ns.EnergyStorageEnv, store(15.)), ("5b", ns.EnergyStorageEnv, store(30.)),
+                  ("20c", ns.EnergyStorageEnv, store(30.)), ("10a", ns.EnergyStorageEnv, store(20.)),
+                  ("7b", ns.EnergyStorageEnv, store(35.)), ("4a", ns.PVEnv, pv(80.))]
+        agents = [{"name": f"a{i}", "bus": bus, "cls": cls, "config": cfg}
+                  for i, (bus, cls, cfg) in enumerate(roster)]
+    return {"common_config": {"start_time": "08-12-2021 00:00:00", "end_time": "08-13-2021 00:00:00",
+                              "control_timedelta": pd.Timedelta(300, "s")},
+            "pf_config": {"cls": ns.OpenDSSSolver,
+                          "config": {"feeder_file": path, "loadshape_file": LOADSHAPE,
+                                     "system_load_rescale_factor": load_factor}},
+            "agents": agents}
 
 
 def band(f):

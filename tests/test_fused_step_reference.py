@@ -76,32 +76,32 @@ def _env(ns, cfg, hook, **kw):
         return cls(**cfg, **kw)
 
 
-def _check_voltages(env, u, v, row, tol, t, label):
-    """Device voltages of one step against the float64 reference: u [nb, E] branch voltages,
-    v [nn, E] node magnitudes; ``row`` = the node whose magnitude the float64 row sweep gives
-    (hook runs; None otherwise).  Returns the largest errors (all nodes, the row, u)."""
+def _check_voltages(env, u, v, row, tol, t, label, cols=slice(None)):
+    """Device voltages of one step against the float64 reference: u [nb, E'] branch voltages,
+    v [nn, E'] node magnitudes of the envs ``cols``; ``row`` = the node whose magnitude the float64
+    row sweep gives (hook runs; None otherwise).  Returns the largest errors (all nodes, the row, u)."""
     vtol, rtol, utol = tol
     nb = env.pf_solver.feeder.nb
     msg = f"{label}, step {t}"
-    got = env.get_field(N.FIELD_VOLTAGES).cpu().numpy()
+    got = env.get_field(N.FIELD_VOLTAGES)[:, cols].cpu().numpy()
     np.testing.assert_allclose(got, v, rtol=0, atol=vtol, err_msg=f"node voltages, {msg}")
     if row is not None:
         np.testing.assert_allclose(got[row], v[row], rtol=0, atol=rtol, err_msg=f"float64 row, {msg}")
-    np.testing.assert_allclose(env.get_field(N.FIELD_VMIN).cpu().numpy(), v.min(axis=0), rtol=0,
+    np.testing.assert_allclose(env.get_field(N.FIELD_VMIN)[cols].cpu().numpy(), v.min(axis=0), rtol=0,
                                atol=vtol, err_msg=f"vmin, {msg}")
-    np.testing.assert_allclose(env.get_field(N.FIELD_VMAX).cpu().numpy(), v.max(axis=0), rtol=0,
+    np.testing.assert_allclose(env.get_field(N.FIELD_VMAX)[cols].cpu().numpy(), v.max(axis=0), rtol=0,
                                atol=vtol, err_msg=f"vmax, {msg}")
-    vbus = env.get_field(N.FIELD_VBUS).cpu().numpy()
+    vbus = env.get_field(N.FIELD_VBUS)[:, cols].cpu().numpy()
     for a, rec in enumerate(env._agent_recs):
         want = v[rec.bus_node] if rec.bus_node >= 0 else np.ones(v.shape[1])
         at = rtol if rec.bus_node == row else vtol
         np.testing.assert_allclose(vbus[a], want, rtol=0, atol=at, err_msg=f"bus voltage of agent {a}, {msg}")
-    ps = env.get_field(N.FIELD_PF_STATE).cpu().numpy()
-    np.testing.assert_allclose(ps[:nb, :, 0] + 1j * ps[:nb, :, 1], u, rtol=0, atol=utol,
+    ps = env.get_field(N.FIELD_PF_STATE)[:nb, cols].cpu().numpy()
+    np.testing.assert_allclose(ps[..., 0] + 1j * ps[..., 1], u, rtol=0, atol=utol,
                                err_msg=f"branch voltages, {msg}")
-    assert int(env.get_field(N.FIELD_PF_ITERS).min()) > 0, f"a power flow did not converge, {msg}"
+    assert int(env.get_field(N.FIELD_PF_ITERS)[cols].min()) > 0, f"a power flow did not converge, {msg}"
     return (np.abs(got - v).max(), 0.0 if row is None else np.abs(got[row] - v[row]).max(),
-            np.abs(ps[:nb, :, 0] + 1j * ps[:nb, :, 1] - u).max())
+            np.abs(ps[..., 0] + 1j * ps[..., 1] - u).max())
 
 
 @pytest.mark.parametrize("hook", [True, False], ids=["hook", "nohook"])
