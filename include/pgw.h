@@ -10,7 +10,8 @@
  * Conventions
  *   - Every per-env array is "rows x E" with the env index fastest varying
  *     (structure of arrays): element (row, e) lives at  ptr[row * E + e].
- *   - All floating point is IEEE double (the reference computes in float64).
+ *   - All floating point is IEEE double (the reference computes in float64); the *_f32
+ *     entry points take float actions and observations instead (computed in double).
  *   - Buffers passed to pgw_reset / pgw_step / pgw_get are DEVICE pointers owned
  *     by the caller (e.g. torch tensors); the *_host variants take HOST pointers
  *     and perform the copies themselves.
@@ -260,6 +261,17 @@ int pgw_reset_host(pgw_env* env, const double* init_soc, double* obs, void* cuda
 int pgw_step_host(pgw_env* env, const double* actions, double* obs, double* rew,
                   uint8_t* done, void* cuda_stream);
 
+/* Float32 I/O: the same four calls with float actions [act_dim][E] and float observations
+ * [obs_dim][E].  The arithmetic is unchanged (float64): actions are widened where they are read,
+ * observations rounded to nearest where they are stored; init_soc, rewards and done flags keep
+ * their types.  A handle may be driven in both forms; pgw_step keeps one captured graph per form. */
+int pgw_reset_f32(pgw_env* env, const double* init_soc, float* obs, void* cuda_stream);
+int pgw_step_f32(pgw_env* env, const float* actions, float* obs, double* rew, uint8_t* done,
+                 void* cuda_stream);
+int pgw_reset_host_f32(pgw_env* env, const double* init_soc, float* obs, void* cuda_stream);
+int pgw_step_host_f32(pgw_env* env, const float* actions, float* obs, double* rew, uint8_t* done,
+                      void* cuda_stream);
+
 /* Stand-alone batched power flow on the handle's feeder: PowerFlowSolver.calculate_power_flow
  * (gridworld/distribution_system/powerflow.py:20-39) used without an env, as in
  * tests/distribution_system/test_opendss.py:7-16.  load_kw / load_kvar are device
@@ -302,8 +314,9 @@ int pgw_stats(pgw_env* env, double* out, void* cuda_stream);
 int pgw_clock(const pgw_env* env);
 /* Number of kernels this handle has launched since creation (bench accounting). */
 long long pgw_launch_count(const pgw_env* env);
-/* CUDA graphs captured and instantiated since creation: pgw_step keeps ONE per handle however many
- * different caller buffers it sees; pgw_step_host one per set of host buffers (at most 8). */
+/* CUDA graphs captured and instantiated since creation: pgw_step keeps ONE per handle and I/O form
+ * (pgw_step / pgw_step_f32) however many different caller buffers it sees; pgw_step_host one per set
+ * of host buffers and I/O form (at most 8). */
 long long pgw_graph_captures(const pgw_env* env);
 /* Resets taken so far.  The first reset of a handle initialises the state that the reference keeps
  * across episodes (Home-Steward meta state and storage cost, gridworld/base_hs.py:53-61); a

@@ -95,6 +95,17 @@ SYMBOLS = {
     "pgw_abi_version": (C.c_int, []),
 }
 
+# the float32 I/O forms of reset / step (include/pgw.h, names ending in _f32).  Kept apart from SYMBOLS on
+# purpose: tests/test_abi.py checks SYMBOLS against the declarations it parses from pgw.h with the pattern
+# pgw_[a-z_]+, which does not match names with digits; tests/test_io_f32_cpu.py checks this table.
+# lib() binds both.
+SYMBOLS_F32 = {
+    "pgw_reset_f32": (C.c_int, [_vp, _vp, _vp, _vp]),
+    "pgw_step_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+    "pgw_reset_host_f32": (C.c_int, [_vp, _vp, _vp, _vp]),
+    "pgw_step_host_f32": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
+}
+
 _lib = None
 
 
@@ -111,7 +122,7 @@ def lib():
                 f"{LIB_PATH} is missing: build it with powergridworld_b200/csrc/build.sh "
                 "(there is no CPU fallback)")
         h = C.CDLL(LIB_PATH)
-        for name, (res, args) in SYMBOLS.items():
+        for name, (res, args) in {**SYMBOLS, **SYMBOLS_F32}.items():
             fn = getattr(h, name)          # AttributeError if the export is missing
             fn.restype = res
             fn.argtypes = args

@@ -48,6 +48,15 @@ if _gym is not None and hasattr(_gym, "vector") and hasattr(_gym.vector, "Vector
     _VectorBase = _gym.vector.VectorEnv
 
 
+def _with_dtype(space, dtype):
+    """``space`` with every ``Box`` in the element type ``dtype`` (the env's ``io_dtype``)."""
+    if isinstance(space, dict):
+        return type(space)({k: _with_dtype(v, dtype) for k, v in space.items()})
+    if isinstance(space, spaces.Box) and space.dtype != dtype:
+        return spaces.Box(space.low, space.high, shape=space.shape, dtype=dtype)
+    return space
+
+
 def to_gym_space(space):
     """``spaces.Box`` / ``spaces.Dict`` (and plain dicts of them) as gymnasium / gym spaces; the
     argument itself when neither library is installed."""
@@ -113,7 +122,9 @@ class BatchedJointVectorEnv(_VectorBase):
     All instances of a handle reach their last step together (termination is a function of the
     step count), so autoreset happens for the whole batch: the step that ends the episode returns
     the first observation of the next one and the final one under ``infos["final_observation"]``.
-    Every step goes through ``step_host``: actions and results cross PCIe inside the call."""
+    Every step goes through ``step_host``: actions and results cross PCIe inside the call.
+    ``io_dtype="float32"`` (passed on to the env) makes the spaces, actions and observations
+    float32; rewards stay float64."""
 
     def __init__(self, config: dict = None, num_envs: int = 1, **kwargs):
         cfg = dict(config or {}, **kwargs)
@@ -137,11 +148,12 @@ class BatchedJointVectorEnv(_VectorBase):
             a0 = min(c._slot["act"][0] for c in comps)
             self.agent_obs_slices[ag.name] = slice(o0, o0 + sum(c._slot["obs"][1] for c in comps))
             self.agent_act_slices[ag.name] = slice(a0, a0 + sum(c._slot["act"][1] for c in comps))
-        self.single_observation_space = to_gym_space(spaces.Box(lo, hi, dtype=np.float64))
-        self.single_action_space = to_gym_space(spaces.Box(alo, ahi, dtype=np.float64))
+        dt = np.dtype(e.io_dtype)
+        self.single_observation_space = to_gym_space(spaces.Box(lo, hi, dtype=dt))
+        self.single_action_space = to_gym_space(spaces.Box(alo, ahi, dtype=dt))
         rep = lambda a: np.broadcast_to(a, (self.num_envs,) + a.shape).copy()
-        self.observation_space = to_gym_space(spaces.Box(rep(lo), rep(hi), dtype=np.float64))
-        self.action_space = to_gym_space(spaces.Box(rep(alo), rep(ahi), dtype=np.float64))
+        self.observation_space = to_gym_space(spaces.Box(rep(lo), rep(hi), dtype=dt))
+        self.action_space = to_gym_space(spaces.Box(rep(alo), rep(ahi), dtype=dt))
         self._act = None
         self.episodes = 0
 
@@ -153,7 +165,7 @@ class BatchedJointVectorEnv(_VectorBase):
 
     def step(self, actions):
         e = self.env
-        actions = np.asarray(actions, dtype=np.float64)
+        actions = np.asarray(actions, dtype=e.io_dtype)
         if actions.shape != (self.num_envs, e.act_dim):
             raise ValueError(f"actions must be [{self.num_envs}, {e.act_dim}]")
         if self._act is None:
@@ -194,8 +206,9 @@ class RLlibBatchedBaseEnv(_BaseEnvBase):
         self.num_envs = int(num_envs)
         self.gymnasium_api = bool(gymnasium_api)
         e = self.env
-        self.observation_space = to_gym_space(e.observation_space)
-        self.action_space = to_gym_space(e.action_space)
+        dt = np.dtype(e.io_dtype)                       # the spaces of the host-buffer step's arrays
+        self.observation_space = to_gym_space(_with_dtype(e.observation_space, dt))
+        self.action_space = to_gym_space(_with_dtype(e.action_space, dt))
         # (agent, component or None, first row, rows) of the flat layouts
         self._obs_items, self._act_items = [], []
         for ag in e.agents:
@@ -223,7 +236,7 @@ class RLlibBatchedBaseEnv(_BaseEnvBase):
     def _fill_actions(self, buf, i, action):
         for agent, comp, a0, n in self._act_items:
             a = action[agent] if comp is None else action[agent][comp]
-            buf[a0:a0 + n, i] = np.asarray(a, dtype=np.float64).reshape(n)
+            buf[a0:a0 + n, i] = np.asarray(a, dtype=buf.dtype).reshape(n)
 
     # ---- BaseEnv
     def poll(self):

@@ -110,8 +110,9 @@ struct pgw_env {
   bool tc2_tol_set = false;             // PGW_OPT_PF_TC_TOL_NANO was given: the polish option leaves tol alone
   pgw::Tc2Consts tc2c{};
   pgw::Tc2Polish tc2p{};
-  // The captured CUDA graph of a step: ONE per handle; its kernel nodes are re-pointed at the
-  // caller's buffers when those change (kind: 0 fused step, 1 components, 2 power flow)
+  // The captured CUDA graph of a step: ONE per handle and I/O form (float64 / float32 actions and
+  // observations, [io32]); its kernel nodes are re-pointed at the caller's buffers when those change
+  // (kind: 0 fused step, 1 components, 2 power flow)
   struct StepGraph {
     cudaGraph_t graph = nullptr;
     cudaGraphExec_t exec = nullptr;
@@ -126,10 +127,11 @@ struct pgw_env {
       exec = nullptr; graph = nullptr; num_nodes = 0;
     }
   };
-  StepGraph step_graph;
-  // graphs of the pipelined host-buffer step, keyed by the host pointers (memcpy nodes)
+  StepGraph step_graph[2];
+  // graphs of the pipelined host-buffer step, keyed by the host pointers (memcpy nodes) and I/O form
   struct HostGraph {
     const void *actions, *obs, *rew, *done;
+    bool io32;
     cudaGraphExec_t exec;
   };
   std::vector<HostGraph> host_graphs;
@@ -143,7 +145,8 @@ struct pgw_env {
   cudaStream_t chunk_stream[kMaxChunks] = {};
   cudaEvent_t ev_fork = nullptr, ev_join[kMaxChunks] = {};
   void drop_graphs() {
-    step_graph.destroy();
+    step_graph[0].destroy();
+    step_graph[1].destroy();
     for (auto& g : host_graphs) cudaGraphExecDestroy(g.exec);
     host_graphs.clear();
   }
@@ -165,6 +168,7 @@ struct pgw_env {
   long long* phase_clk = nullptr;       // PGW_PHASE_TIMERS builds (tools/phase_probe.py)
   // staging for the *_host entry points
   double *h_act = nullptr, *h_obs = nullptr, *h_rew = nullptr, *h_soc = nullptr;
+  float *h_act32 = nullptr, *h_obs32 = nullptr;   // float32 I/O (the *_f32 entry points)
   uint8_t* h_done = nullptr;
   std::vector<void*> owned;
   // optional per-kernel timing (pgw_set_timing)
@@ -871,6 +875,8 @@ int pgw_destroy(pgw_env* env) {
   if (!env) return PGW_OK;
   if (env->h_act) cudaFree(env->h_act);
   if (env->h_obs) cudaFree(env->h_obs);
+  if (env->h_act32) cudaFree(env->h_act32);
+  if (env->h_obs32) cudaFree(env->h_obs32);
   if (env->h_rew) cudaFree(env->h_rew);
   if (env->h_soc) cudaFree(env->h_soc);
   if (env->h_done) cudaFree(env->h_done);
@@ -946,7 +952,8 @@ static int smem_for_events(const pgw_env* env, bool reset = false) {
          ((reset ? env->need_scratch_reset : env->need_scratch) ? 35 * 64 * 8 : 0);
 }
 
-int pgw_reset(pgw_env* env, const double* init_soc, double* obs, void* cuda_stream) {
+// io32: obs is a float array (pgw_reset_f32), else double
+static int reset_impl(pgw_env* env, const double* init_soc, void* obs, bool io32, void* cuda_stream) {
   if (!env || !obs) return fail(PGW_ERR_INVALID, "null argument");
   cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
   PGW_CUDA(cudaMemsetAsync(env->d_clock, 0, sizeof(int), s));
@@ -959,7 +966,7 @@ int pgw_reset(pgw_env* env, const double* init_soc, double* obs, void* cuda_stre
     ++env->launches;
   }
   pgw::CompParams cp = comp_params(env);
-  cp.event_mode = 0; cp.advance_clock = 0; cp.init_soc = init_soc; cp.obs = obs;
+  cp.event_mode = 0; cp.advance_clock = 0; cp.init_soc = init_soc; cp.obs = obs; cp.io32 = io32 ? 1 : 0;
   cp.clip_init_soc = env->clip_init_soc ? 1 : 0;
   cp.first_reset = env->resets == 0 ? 1 : 0;
   ++env->resets;
@@ -969,13 +976,22 @@ int pgw_reset(pgw_env* env, const double* init_soc, double* obs, void* cuda_stre
   return PGW_OK;
 }
 
+int pgw_reset(pgw_env* env, const double* init_soc, double* obs, void* cuda_stream) {
+  return reset_impl(env, init_soc, obs, false, cuda_stream);
+}
+
+int pgw_reset_f32(pgw_env* env, const double* init_soc, float* obs, void* cuda_stream) {
+  return reset_impl(env, init_soc, obs, true, cuda_stream);
+}
+
 // ---- launch parameters of the kernels of one step over the envs [e_lo, e_hi)
-static pgw::CompParams step_comp_params(pgw_env* env, const double* actions, double* obs, double* rew,
-                                        uint8_t* done, int e_lo, int e_hi, int chunks, int pdl_trigger) {
+static pgw::CompParams step_comp_params(pgw_env* env, const void* actions, void* obs, double* rew,
+                                        uint8_t* done, bool io32, int e_lo, int e_hi, int chunks,
+                                        int pdl_trigger) {
   pgw::CompParams cp = comp_params(env);
   const bool hook = env->has_feeder && env->punit != 0.0;   // power flow finishes the rewards
   cp.event_mode = 1; cp.advance_clock = env->has_feeder ? 0 : 1; cp.owns_reward = hook ? 0 : 1;
-  cp.actions = actions; cp.obs = obs; cp.rew = rew; cp.done = done;
+  cp.actions = actions; cp.obs = obs; cp.rew = rew; cp.done = done; cp.io32 = io32 ? 1 : 0;
   cp.pdl_trigger = pdl_trigger;
   cp.e_lo = e_lo; cp.e_hi = e_hi; cp.tickets = (unsigned int)(env->num_ctas * chunks);
   return cp;
@@ -1022,12 +1038,12 @@ static int fused_grid(int envs) {
 
 // `tickets` = CTAs of all the launches that make up the step (the CTA that takes the last ticket
 // advances the clock); 0 = this launch is the whole step.
-static pgw::FusedParams step_fused_params(pgw_env* env, const double* actions, double* obs, double* rew,
-                                          uint8_t* done, int e_lo, int e_hi, unsigned int tickets,
+static pgw::FusedParams step_fused_params(pgw_env* env, const void* actions, void* obs, double* rew,
+                                          uint8_t* done, bool io32, int e_lo, int e_hi, unsigned int tickets,
                                           int stagger = 0, int event = -1) {
   pgw::FusedParams P{};
   P.event = event;
-  P.c = step_comp_params(env, actions, obs, rew, done, e_lo, e_hi, 1, 0);
+  P.c = step_comp_params(env, actions, obs, rew, done, io32, e_lo, e_hi, 1, 0);
   P.f = step_pf_params(env, rew, e_lo, e_hi, 1u, false);
   P.C = env->C; P.act_dim = env->act_dim; P.sd_rows = env->sd_rows; P.e_lo = e_lo; P.e_hi = e_hi;
   P.tickets = tickets ? tickets : (unsigned int)fused_grid(e_hi - e_lo);
@@ -1053,13 +1069,14 @@ static unsigned int step_pf_tickets(pgw_env* env, const int* bounds, int chunks)
   return n;
 }
 
-static int enqueue_step(pgw_env* env, const double* actions, double* obs, double* rew,
-                        uint8_t* done, cudaStream_t s, bool timed, int e_lo = 0, int e_hi = -1,
+static int enqueue_step(pgw_env* env, const void* actions, void* obs, double* rew,
+                        uint8_t* done, bool io32, cudaStream_t s, bool timed, int e_lo = 0, int e_hi = -1,
                         int chunks = 1, unsigned int pf_tickets = 0u, int stagger = 0, int event = -1) {
   if (e_hi < 0) e_hi = env->E;
   if (use_fused(env)) {
     if (timed) PGW_CUDA(cudaEventRecord(env->next_event(), s));
-    const pgw::FusedParams P = step_fused_params(env, actions, obs, rew, done, e_lo, e_hi, pf_tickets, stagger, event);
+    const pgw::FusedParams P = step_fused_params(env, actions, obs, rew, done, io32, e_lo, e_hi, pf_tickets, stagger,
+                                                 event);
     PGW_CUDA(pgw::launch_step_fused(P, fused_grid(e_hi - e_lo), s));
     if (timed) {                                       // one kernel: reported in the component slot
       PGW_CUDA(cudaEventRecord(env->next_event(), s));
@@ -1069,7 +1086,7 @@ static int enqueue_step(pgw_env* env, const double* actions, double* obs, double
   }
   const int pdl = chunks == 1 ? pdl_trigger_mode(env, timed) : 0;
   if (timed) PGW_CUDA(cudaEventRecord(env->next_event(), s));
-  PGW_CUDA(pgw::launch_components(step_comp_params(env, actions, obs, rew, done, e_lo, e_hi, chunks, pdl),
+  PGW_CUDA(pgw::launch_components(step_comp_params(env, actions, obs, rew, done, io32, e_lo, e_hi, chunks, pdl),
                                   smem_for_events(env), s));
   if (timed) PGW_CUDA(cudaEventRecord(env->next_event(), s));
   if (env->has_feeder)
@@ -1083,9 +1100,9 @@ static int step_kernels(const pgw_env* env) { return use_fused(env) ? 1 : (env->
 // Re-point the kernel nodes of the captured step graph at another set of caller buffers
 // (cudaGraphExecKernelNodeSetParams: no re-capture, no re-instantiation; a policy loop that
 // hands in a fresh action tensor every step replays the same executable graph).
-static int retarget_step_graph(pgw_env* env, const double* actions, double* obs, double* rew,
-                               uint8_t* done, int event) {
-  pgw_env::StepGraph& g = env->step_graph;
+static int retarget_step_graph(pgw_env* env, const void* actions, void* obs, double* rew,
+                               uint8_t* done, bool io32, int event) {
+  pgw_env::StepGraph& g = env->step_graph[io32];
   for (int i = 0; i < g.num_nodes; ++i) {
     cudaKernelNodeParams np = g.params[i];
     void* args[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -1094,11 +1111,11 @@ static int retarget_step_graph(pgw_env* env, const double* actions, double* obs,
     pgw::CompParams cp;
     pgw::PfParams pf;
     if (g.kind[i] == 0) {
-      fp = step_fused_params(env, actions, obs, rew, done, 0, env->E, 0u, 0, event);
+      fp = step_fused_params(env, actions, obs, rew, done, io32, 0, env->E, 0u, 0, event);
       args[0] = &fp;
       g.has_event = event >= 0;
     } else if (g.kind[i] == 1) {
-      cp = step_comp_params(env, actions, obs, rew, done, 0, env->E, 1, g.pdl);
+      cp = step_comp_params(env, actions, obs, rew, done, io32, 0, env->E, 1, g.pdl);
       args[0] = &cp;
     } else {
       pf = step_pf_params(env, rew, 0, env->E, 0u, g.pdl != 0);
@@ -1112,13 +1129,13 @@ static int retarget_step_graph(pgw_env* env, const double* actions, double* obs,
   return PGW_OK;
 }
 
-static int capture_step_graph(pgw_env* env, const double* actions, double* obs, double* rew,
-                              uint8_t* done, cudaStream_t s) {
-  pgw_env::StepGraph& g = env->step_graph;
+static int capture_step_graph(pgw_env* env, const void* actions, void* obs, double* rew,
+                              uint8_t* done, bool io32, cudaStream_t s) {
+  pgw_env::StepGraph& g = env->step_graph[io32];
   g.destroy();
   g.pdl = pdl_trigger_mode(env, false);
   PGW_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-  int rc = enqueue_step(env, actions, obs, rew, done, s, false);
+  int rc = enqueue_step(env, actions, obs, rew, done, io32, s, false);
   cudaError_t ce = cudaStreamEndCapture(s, &g.graph);
   if (rc != PGW_OK) { g.destroy(); return rc; }
   if (ce != cudaSuccess) {
@@ -1152,8 +1169,8 @@ static int capture_step_graph(pgw_env* env, const double* actions, double* obs, 
   return PGW_OK;
 }
 
-int pgw_step(pgw_env* env, const double* actions, double* obs, double* rew, uint8_t* done,
-             void* cuda_stream) {
+static int step_impl(pgw_env* env, const void* actions, void* obs, double* rew, uint8_t* done, bool io32,
+                     void* cuda_stream) {
   if (!env || !actions || !obs || !rew || !done) return fail(PGW_ERR_INVALID, "null argument");
   if (env->clock < 0) return fail(PGW_ERR_STATE, "pgw_step before pgw_reset");
   if (env->clock + 1 >= env->num_events)
@@ -1167,22 +1184,22 @@ int pgw_step(pgw_env* env, const double* actions, double* obs, double* rew, uint
   const bool graphable = env->use_graphs && !env->timing && cap == cudaStreamCaptureStatusNone &&
                          s != nullptr;
   if (graphable) {
-    pgw_env::StepGraph& g = env->step_graph;
+    pgw_env::StepGraph& g = env->step_graph[io32];
     int rc = PGW_OK;
-    if (!g.exec) rc = capture_step_graph(env, actions, obs, rew, done, s);
+    if (!g.exec) rc = capture_step_graph(env, actions, obs, rew, done, io32, s);
     else if (g.actions != actions || g.obs != obs || g.rew != rew || g.done != done)
       // the node parameters are rewritten anyway: the step's event index rides along and the
       // fused kernel skips its read of the device clock
-      rc = retarget_step_graph(env, actions, obs, rew, done, env->clock + 1);
+      rc = retarget_step_graph(env, actions, obs, rew, done, io32, env->clock + 1);
     else if (g.has_event)                              // same buffers again: back to the device clock
-      rc = retarget_step_graph(env, actions, obs, rew, done, -1);
+      rc = retarget_step_graph(env, actions, obs, rew, done, io32, -1);
     if (rc != PGW_OK) return rc;
     PGW_CUDA(cudaGraphLaunch(g.exec, s));
   } else {
     // direct launches know the event index; a launch recorded into the CALLER's capture is
     // replayed with frozen parameters and has to read the device clock
     const int event = cap == cudaStreamCaptureStatusNone ? env->clock + 1 : -1;
-    int rc = enqueue_step(env, actions, obs, rew, done, s, env->timing, 0, -1, 1, 0u, 0, event);
+    int rc = enqueue_step(env, actions, obs, rew, done, io32, s, env->timing, 0, -1, 1, 0u, 0, event);
     if (rc != PGW_OK) return rc;
   }
   env->launches += step_kernels(env);
@@ -1190,10 +1207,26 @@ int pgw_step(pgw_env* env, const double* actions, double* obs, double* rew, uint
   return PGW_OK;
 }
 
-static int ensure_staging(pgw_env* env) {
+int pgw_step(pgw_env* env, const double* actions, double* obs, double* rew, uint8_t* done,
+             void* cuda_stream) {
+  return step_impl(env, actions, obs, rew, done, false, cuda_stream);
+}
+
+int pgw_step_f32(pgw_env* env, const float* actions, float* obs, double* rew, uint8_t* done,
+                 void* cuda_stream) {
+  return step_impl(env, actions, obs, rew, done, true, cuda_stream);
+}
+
+// device staging of the host-buffer entry points: actions / observations in the I/O form's element type
+static int ensure_staging(pgw_env* env, bool io32) {
   const size_t E = (size_t)env->E;
-  if (!env->h_act) PGW_CUDA(cudaMalloc(&env->h_act, (size_t)env->act_dim * E * 8));
-  if (!env->h_obs) PGW_CUDA(cudaMalloc(&env->h_obs, (size_t)env->obs_dim * E * 8));
+  if (io32) {
+    if (!env->h_act32) PGW_CUDA(cudaMalloc(&env->h_act32, (size_t)env->act_dim * E * 4));
+    if (!env->h_obs32) PGW_CUDA(cudaMalloc(&env->h_obs32, (size_t)env->obs_dim * E * 4));
+  } else {
+    if (!env->h_act) PGW_CUDA(cudaMalloc(&env->h_act, (size_t)env->act_dim * E * 8));
+    if (!env->h_obs) PGW_CUDA(cudaMalloc(&env->h_obs, (size_t)env->obs_dim * E * 8));
+  }
   if (!env->h_rew) PGW_CUDA(cudaMalloc(&env->h_rew, (size_t)env->A * E * 8));
   if (!env->h_done) PGW_CUDA(cudaMalloc(&env->h_done, E));
   if (!env->h_soc && env->num_storage)
@@ -1201,20 +1234,29 @@ static int ensure_staging(pgw_env* env) {
   return PGW_OK;
 }
 
-int pgw_reset_host(pgw_env* env, const double* init_soc, double* obs, void* cuda_stream) {
+static int reset_host_impl(pgw_env* env, const double* init_soc, void* obs, bool io32, void* cuda_stream) {
   if (!env || !obs) return fail(PGW_ERR_INVALID, "null argument");
-  int rc = ensure_staging(env);
+  int rc = ensure_staging(env, io32);
   if (rc) return rc;
   cudaStream_t s = static_cast<cudaStream_t>(cuda_stream);
   const size_t E = (size_t)env->E;
   if (init_soc && env->num_storage)
     PGW_CUDA(cudaMemcpyAsync(env->h_soc, init_soc, (size_t)env->num_storage * E * 8,
                              cudaMemcpyHostToDevice, s));
-  rc = pgw_reset(env, (init_soc && env->num_storage) ? env->h_soc : nullptr, env->h_obs, s);
+  void* stage = io32 ? (void*)env->h_obs32 : (void*)env->h_obs;
+  rc = reset_impl(env, (init_soc && env->num_storage) ? env->h_soc : nullptr, stage, io32, s);
   if (rc) return rc;
-  PGW_CUDA(cudaMemcpyAsync(obs, env->h_obs, (size_t)env->obs_dim * E * 8, cudaMemcpyDeviceToHost, s));
+  PGW_CUDA(cudaMemcpyAsync(obs, stage, (size_t)env->obs_dim * E * (io32 ? 4 : 8), cudaMemcpyDeviceToHost, s));
   PGW_CUDA(cudaStreamSynchronize(s));
   return PGW_OK;
+}
+
+int pgw_reset_host(pgw_env* env, const double* init_soc, double* obs, void* cuda_stream) {
+  return reset_host_impl(env, init_soc, obs, false, cuda_stream);
+}
+
+int pgw_reset_host_f32(pgw_env* env, const double* init_soc, float* obs, void* cuda_stream) {
+  return reset_host_impl(env, init_soc, obs, true, cuda_stream);
 }
 
 // ---- end-to-end step with host buffers, pipelined over env chunks.
@@ -1223,12 +1265,12 @@ int pgw_reset_host(pgw_env* env, const double* init_soc, double* obs, void* cuda
 // so that the copy-in of chunk k+1, the kernels of chunk k and the copy-out of chunk k-1 overlap
 // (PCIe is full duplex, the copy engines are independent of the SMs).  The whole fork-join is
 // captured once per set of host buffers and replayed as one graph launch.
-static int host_chunks(const pgw_env* env) {
+static int host_chunks(const pgw_env* env, bool io32) {
   if (env->timing || (env->has_feeder && env->pf_kernel == 1)) return 1;   // kernel 1 has no env ranges
   if (env->host_chunks > 0) return std::min(env->host_chunks, pgw_env::kMaxChunks);
   // Every copy costs ~8 us of fixed latency on top of its bytes (measured, C1: 94 us per step
   // with one chunk, 120 with four): chunks pay off only when a chunk's copy-out is several MB
-  const size_t out = (size_t)env->obs_dim * (size_t)env->E * 8;
+  const size_t out = (size_t)env->obs_dim * (size_t)env->E * (io32 ? 4 : 8);
   return out >= ((size_t)32 << 20) ? 4 : 1;
 }
 
@@ -1247,28 +1289,30 @@ static void* device_view(pgw_env* env, const void* host) {
   return dev;
 }
 
-static int enqueue_host_step(pgw_env* env, const double* actions, double* obs, double* rew,
-                             uint8_t* done, cudaStream_t s) {
-  const int E = env->E, nch = host_chunks(env);
+static int enqueue_host_step(pgw_env* env, const void* actions, void* obs, double* rew,
+                             uint8_t* done, bool io32, cudaStream_t s) {
+  const int E = env->E, nch = host_chunks(env, io32);
   int bounds[pgw_env::kMaxChunks + 1];
   const int per = ((E + nch - 1) / nch + 127) / 128 * 128;          // whole 128-env tiles
   for (int k = 0; k <= nch; ++k) bounds[k] = std::min(E, k * per);
   const unsigned int tickets = env->has_feeder ? step_pf_tickets(env, bounds, nch) : 0u;
-  const size_t pitch = (size_t)E * 8;
+  const size_t pitch = (size_t)E * 8, esz = io32 ? 4 : 8, io_pitch = (size_t)E * esz;
+  unsigned char* act_stage = io32 ? (unsigned char*)env->h_act32 : (unsigned char*)env->h_act;
+  unsigned char* obs_stage = io32 ? (unsigned char*)env->h_obs32 : (unsigned char*)env->h_obs;
   if (nch > 1) PGW_CUDA(cudaEventRecord(env->ev_fork, s));
   for (int k = 0; k < nch; ++k) {
     const int e0 = bounds[k], e1 = bounds[k + 1];
     if (e1 <= e0) continue;
     cudaStream_t ck = nch > 1 ? env->chunk_stream[k] : s;
     if (nch > 1) PGW_CUDA(cudaStreamWaitEvent(ck, env->ev_fork, 0));
-    const size_t w8 = (size_t)(e1 - e0) * 8;
-    PGW_CUDA(cudaMemcpy2DAsync(env->h_act + e0, pitch, actions + e0, pitch, w8, (size_t)env->act_dim,
-                               cudaMemcpyHostToDevice, ck));
-    int rc = enqueue_step(env, env->h_act, env->h_obs, env->h_rew, env->h_done, ck, env->timing, e0, e1,
+    const size_t w8 = (size_t)(e1 - e0) * 8, wio = (size_t)(e1 - e0) * esz, o0 = (size_t)e0 * esz;
+    PGW_CUDA(cudaMemcpy2DAsync(act_stage + o0, io_pitch, static_cast<const unsigned char*>(actions) + o0, io_pitch,
+                               wio, (size_t)env->act_dim, cudaMemcpyHostToDevice, ck));
+    int rc = enqueue_step(env, act_stage, obs_stage, env->h_rew, env->h_done, io32, ck, env->timing, e0, e1,
                           nch, tickets);
     if (rc) return rc;
-    PGW_CUDA(cudaMemcpy2DAsync(obs + e0, pitch, env->h_obs + e0, pitch, w8, (size_t)env->obs_dim,
-                               cudaMemcpyDeviceToHost, ck));
+    PGW_CUDA(cudaMemcpy2DAsync(static_cast<unsigned char*>(obs) + o0, io_pitch, obs_stage + o0, io_pitch, wio,
+                               (size_t)env->obs_dim, cudaMemcpyDeviceToHost, ck));
     PGW_CUDA(cudaMemcpy2DAsync(rew + e0, pitch, env->h_rew + e0, pitch, w8, (size_t)env->A,
                                cudaMemcpyDeviceToHost, ck));
     PGW_CUDA(cudaMemcpyAsync(done + e0, env->h_done + e0, (size_t)(e1 - e0), cudaMemcpyDeviceToHost, ck));
@@ -1293,14 +1337,19 @@ static int zero_copy_chunks(const pgw_env* env) {
   return env->host_chunks > 0 ? std::min(env->host_chunks, pgw_env::kMaxChunks) : 1;
 }
 
-static int enqueue_zero_copy(pgw_env* env, const double* actions, double* obs, double* rew, uint8_t* done,
-                             cudaStream_t s) {
+// float32 actions: 128-byte rows.  Measured on a B200 (1000 W), C1 at 4096 envs, zero-copy step_host, wall us
+// per call (medians of three sessions): 3 cycles per row 51.0, 2: 51.2, 5: 53.0, 10: 57.9, 0: 54.9
+// (profiles/r4_e2e_io_dtype.jsonl, DESIGN.md section 6.0b)
+constexpr int kStaggerPerRowF32 = 3;
+
+static int enqueue_zero_copy(pgw_env* env, const void* actions, void* obs, double* rew, uint8_t* done,
+                             bool io32, cudaStream_t s) {
   const int E = env->E, nch = zero_copy_chunks(env);
   // one tile's actions (act_dim x 256 B) at ~48 GB/s of PCIe reads, in cycles of the 1.965 GHz SM clock
-  int per_row = 10;
+  int per_row = io32 ? kStaggerPerRowF32 : 10;
   if (const char* v = getenv("PGW_STAGGER_CYCLES_PER_ROW")) per_row = atoi(v);   // tuning knob
   const int stagger = env->act_dim * per_row;
-  if (nch == 1) return enqueue_step(env, actions, obs, rew, done, s, false, 0, -1, 1, 0u, stagger);
+  if (nch == 1) return enqueue_step(env, actions, obs, rew, done, io32, s, false, 0, -1, 1, 0u, stagger);
   int bounds[pgw_env::kMaxChunks + 1];
   const int per = ((E + nch - 1) / nch + 31) / 32 * 32;             // whole 32-env tiles
   for (int k = 0; k <= nch; ++k) bounds[k] = std::min(E, k * per);
@@ -1310,7 +1359,7 @@ static int enqueue_zero_copy(pgw_env* env, const double* actions, double* obs, d
   bool first = true;
   for (int k = 0; k < nch; ++k) {
     if (bounds[k + 1] <= bounds[k]) continue;
-    pgw::FusedParams P = step_fused_params(env, actions, obs, rew, done, bounds[k], bounds[k + 1], tickets);
+    pgw::FusedParams P = step_fused_params(env, actions, obs, rew, done, io32, bounds[k], bounds[k + 1], tickets);
     P.pdl_trigger = 1;
     PGW_CUDA(pgw::launch_step_fused(P, fused_grid(bounds[k + 1] - bounds[k]), s, !first));
     first = false;
@@ -1318,7 +1367,7 @@ static int enqueue_zero_copy(pgw_env* env, const double* actions, double* obs, d
   return PGW_OK;
 }
 
-static int zero_copy_step(pgw_env* env, const double* actions, double* obs, double* rew, uint8_t* done,
+static int zero_copy_step(pgw_env* env, const void* actions, void* obs, double* rew, uint8_t* done, bool io32,
                           cudaStream_t s) {
   const int nch = zero_copy_chunks(env);
   if (env->clock < 0) return fail(PGW_ERR_STATE, "pgw_step before pgw_reset");
@@ -1328,25 +1377,25 @@ static int zero_copy_step(pgw_env* env, const double* actions, double* obs, doub
   cudaGraphExec_t exec = nullptr;
   if (env->use_graphs && cap == cudaStreamCaptureStatusNone && s != nullptr) {
     for (auto& g : env->host_graphs)
-      if (g.actions == actions && g.obs == obs && g.rew == rew && g.done == done) exec = g.exec;
+      if (g.actions == actions && g.obs == obs && g.rew == rew && g.done == done && g.io32 == io32) exec = g.exec;
     if (!exec && env->host_graphs.size() < 8) {        // a few pinned buffer sets; beyond: direct
       cudaGraph_t graph = nullptr;
       PGW_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-      int rc = enqueue_zero_copy(env, actions, obs, rew, done, s);
+      int rc = enqueue_zero_copy(env, actions, obs, rew, done, io32, s);
       cudaError_t ce = cudaStreamEndCapture(s, &graph);
       if (rc != PGW_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
       if (ce != cudaSuccess) return fail(PGW_ERR_CUDA, std::string("graph capture: ") + cudaGetErrorString(ce));
       ce = cudaGraphInstantiate(&exec, graph, 0);
       cudaGraphDestroy(graph);
       if (ce != cudaSuccess) return fail(PGW_ERR_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce));
-      env->host_graphs.push_back({actions, obs, rew, done, exec});
+      env->host_graphs.push_back({actions, obs, rew, done, io32, exec});
       ++env->graph_captures;
     }
   }
   if (exec) {
     PGW_CUDA(cudaGraphLaunch(exec, s));
   } else {
-    int rc = enqueue_zero_copy(env, actions, obs, rew, done, s);
+    int rc = enqueue_zero_copy(env, actions, obs, rew, done, io32, s);
     if (rc) return rc;
   }
   env->launches += nch * step_kernels(env);
@@ -1354,8 +1403,8 @@ static int zero_copy_step(pgw_env* env, const double* actions, double* obs, doub
   return PGW_OK;
 }
 
-int pgw_step_host(pgw_env* env, const double* actions, double* obs, double* rew, uint8_t* done,
-                  void* cuda_stream) {
+static int step_host_impl(pgw_env* env, const void* actions, void* obs, double* rew, uint8_t* done, bool io32,
+                          void* cuda_stream) {
   if (!env || !actions || !obs || !rew || !done) return fail(PGW_ERR_INVALID, "null argument");
   if (env->clock < 0) return fail(PGW_ERR_STATE, "pgw_step before pgw_reset");
   if (env->clock + 1 >= env->num_events)
@@ -1372,14 +1421,13 @@ int pgw_step_host(pgw_env* env, const double* actions, double* obs, double* rew,
     void* dr = device_view(env, rew);
     void* dd = device_view(env, done);
     if (da && dobs && dr && dd) {
-      rc = zero_copy_step(env, static_cast<const double*>(da), static_cast<double*>(dobs),
-                          static_cast<double*>(dr), static_cast<uint8_t*>(dd), s);
+      rc = zero_copy_step(env, da, dobs, static_cast<double*>(dr), static_cast<uint8_t*>(dd), io32, s);
       if (rc) return rc;
       PGW_CUDA(cudaStreamSynchronize(s));
       return PGW_OK;
     }
   }
-  rc = ensure_staging(env);
+  rc = ensure_staging(env, io32);
   if (rc) return rc;
   if (!env->ev_fork) {
     PGW_CUDA(cudaEventCreateWithFlags(&env->ev_fork, cudaEventDisableTiming));
@@ -1395,30 +1443,40 @@ int pgw_step_host(pgw_env* env, const double* actions, double* obs, double* rew,
   cudaGraphExec_t exec = nullptr;
   if (graphable) {
     for (auto& g : env->host_graphs)
-      if (g.actions == actions && g.obs == obs && g.rew == rew && g.done == done) exec = g.exec;
+      if (g.actions == actions && g.obs == obs && g.rew == rew && g.done == done && g.io32 == io32) exec = g.exec;
     if (!exec && env->host_graphs.size() < 8) {        // a few pinned buffer sets; beyond: direct
       cudaGraph_t graph = nullptr;
       PGW_CUDA(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-      rc = enqueue_host_step(env, actions, obs, rew, done, s);
+      rc = enqueue_host_step(env, actions, obs, rew, done, io32, s);
       cudaError_t ce = cudaStreamEndCapture(s, &graph);
       if (rc != PGW_OK) { if (graph) cudaGraphDestroy(graph); return rc; }
       if (ce != cudaSuccess) return fail(PGW_ERR_CUDA, std::string("graph capture: ") + cudaGetErrorString(ce));
       ce = cudaGraphInstantiate(&exec, graph, 0);
       cudaGraphDestroy(graph);
       if (ce != cudaSuccess) return fail(PGW_ERR_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce));
-      env->host_graphs.push_back({actions, obs, rew, done, exec});
+      env->host_graphs.push_back({actions, obs, rew, done, io32, exec});
       ++env->graph_captures;
     }
   }
   if (exec) {
     PGW_CUDA(cudaGraphLaunch(exec, s));
-  } else if ((rc = enqueue_host_step(env, actions, obs, rew, done, s))) {
+  } else if ((rc = enqueue_host_step(env, actions, obs, rew, done, io32, s))) {
     return rc;
   }
   PGW_CUDA(cudaStreamSynchronize(s));
-  env->launches += step_kernels(env) * host_chunks(env);
+  env->launches += step_kernels(env) * host_chunks(env, io32);
   ++env->clock;
   return PGW_OK;
+}
+
+int pgw_step_host(pgw_env* env, const double* actions, double* obs, double* rew, uint8_t* done,
+                  void* cuda_stream) {
+  return step_host_impl(env, actions, obs, rew, done, false, cuda_stream);
+}
+
+int pgw_step_host_f32(pgw_env* env, const float* actions, float* obs, double* rew, uint8_t* done,
+                      void* cuda_stream) {
+  return step_host_impl(env, actions, obs, rew, done, true, cuda_stream);
 }
 
 static int field_location(pgw_env* env, int field, void** ptr, size_t* want) {

@@ -47,16 +47,20 @@ struct Scratch {
 };
 constexpr int kScratchDoubles = 35;
 
-// Everything one (env, agent) worker needs; all per-env arrays are rows x E.
-struct AgentIO {
+// Everything one (env, agent) worker needs; all per-env arrays are rows x E.  ActT / ObsT: element
+// types of the caller's action and observation arrays (double, or float for float32 I/O).  The
+// arithmetic is float64 either way: actions are widened exactly where they are read (act_in),
+// observations rounded to nearest where they are stored (obs_val).
+template <class ActT, class ObsT>
+struct AgentIOT {
   Scratch scr;
   int E;
   // The arrays never alias each other; telling the compiler lets it overlap the many
   // independent load -> divide -> store chains of one agent (the kernel is latency bound).
-  const double* PGW_RESTRICT actions;   // [act_dim][aE], env e at column e - ae0 (unused at reset): the
+  const ActT* PGW_RESTRICT actions;     // [act_dim][aE], env e at column e - ae0 (unused at reset): the
   int aE, ae0;                          // caller's [act_dim][E] array (aE = E, ae0 = 0) or a tile of it
                                         // staged in shared memory (step_fused.cu)
-  double* PGW_RESTRICT obs;             // [obs_dim][E]
+  ObsT* PGW_RESTRICT obs;               // [obs_dim][E]
   double* PGW_RESTRICT sd;              // [sd_rows][E]
   uint32_t* PGW_RESTRICT si;            // [si_rows][E]
   const double* PGW_RESTRICT init_soc;  // [num_storage][E] or nullptr (reset only)
@@ -71,13 +75,27 @@ struct AgentIO {
   const double* PGW_RESTRICT drow;      // event row (doubles)
   const int32_t* PGW_RESTRICT irow;     // event row (int32)
 };
+using AgentIO = AgentIOT<double, double>;
 
 PGW_HD double clip(double x, double lo, double hi) { return fmin(fmax(x, lo), hi); }
 
-// action row `row` of env e
-PGW_HD double act_in(const AgentIO& io, int row, int e) {
-  return io.actions[(size_t)row * io.aE + (e - io.ae0)];
+// action row `row` of env e, widened to double (exact for a float)
+template <class IO>
+PGW_HD double act_in(const IO& io, int row, int e) {
+  return (double)io.actions[(size_t)row * io.aE + (e - io.ae0)];
 }
+
+// an observation value in the caller's element type: as computed, or rounded to the nearest float
+PGW_HD double io_round(double v, const double*) { return v; }
+PGW_HD float io_round(double v, const float*) {
+#if defined(__CUDA_ARCH__)
+  return __double2float_rn(v);
+#else
+  return static_cast<float>(v);
+#endif
+}
+template <class IO>
+PGW_HD auto obs_val(const IO& io, double v) { return io_round(v, io.obs); }
 
 // x / d when r = RN(1/d) was computed on the host: one multiply plus one FMA-based
 // correction (Markstein) returns the correctly rounded IEEE quotient, i.e. the same bits
@@ -105,16 +123,18 @@ PGW_HD double storage_obs(const pgw_component& c, const double* dp, double soc) 
   return (c.flags & PGW_F_RESCALE) ? to_scaled(soc, dp[0], dp[1], dp[7]) : soc;
 }
 
-PGW_HD void storage_reset(const pgw_component& c, const AgentIO& io, int e) {
+template <class IO>
+PGW_HD void storage_reset(const pgw_component& c, const IO& io, int e) {
   const double* dp = io.dpar + c.dpar_off;
   double* soc = io.sd + (size_t)c.sd_off * io.E + e;
   const int ord = io.ipar[c.ipar_off];
   const double init = io.init_soc != nullptr ? io.init_soc[(size_t)ord * io.E + e] : dp[6];
   *soc = (io.init_soc != nullptr && !io.clip_init_soc) ? init : clip(init, dp[0], dp[1]);   // :82-89
-  io.obs[(size_t)c.obs_off * io.E + e] = storage_obs(c, dp, *soc);
+  io.obs[(size_t)c.obs_off * io.E + e] = obs_val(io, storage_obs(c, dp, *soc));
 }
 
-PGW_HD void storage_step(const pgw_component& c, const AgentIO& io, int e, double& p_out) {
+template <class IO>
+PGW_HD void storage_step(const pgw_component& c, const IO& io, int e, double& p_out) {
   const double* dp = io.dpar + c.dpar_off;
   const double lo = dp[0], hi = dp[1], eta_c = dp[2], eta_d = dp[3], pmax = dp[4], dt = dp[5];
   const double inv_eta_d = dp[8], inv_dt = dp[9];
@@ -137,22 +157,25 @@ PGW_HD void storage_step(const pgw_component& c, const AgentIO& io, int e, doubl
     soc = fmax(soc, lo);
   }
   *soc_p = soc;
-  io.obs[(size_t)c.obs_off * io.E + e] = storage_obs(c, dp, soc);
+  io.obs[(size_t)c.obs_off * io.E + e] = obs_val(io, storage_obs(c, dp, soc));
   p_out = -p;
 }
 
 // ------------------------------------------------------------------ PV
-PGW_HD void pv_obs(const pgw_component& c, const AgentIO& io, int e, double raw_power) {
+template <class IO>
+PGW_HD void pv_obs(const pgw_component& c, const IO& io, int e, double raw_power) {
   const double* dp = io.dpar + c.dpar_off;
   const bool rs = (c.flags & PGW_F_RESCALE) != 0;
-  io.obs[(size_t)c.obs_off * io.E + e] = rs ? to_scaled(raw_power, dp[0], dp[1], dp[4]) : raw_power;
+  io.obs[(size_t)c.obs_off * io.E + e] =
+      obs_val(io, rs ? to_scaled(raw_power, dp[0], dp[1], dp[4]) : raw_power);
   if (c.flags & PGW_F_GRID_AWARE) {
     const double v = io.vmin[e];
-    io.obs[(size_t)(c.obs_off + 1) * io.E + e] = rs ? to_scaled(v, dp[2], dp[3], dp[5]) : v;
+    io.obs[(size_t)(c.obs_off + 1) * io.E + e] = obs_val(io, rs ? to_scaled(v, dp[2], dp[3], dp[5]) : v);
   }
 }
 
-PGW_HD void pv_step(const pgw_component& c, const AgentIO& io, int e, double& p_out,
+template <class IO>
+PGW_HD void pv_step(const pgw_component& c, const IO& io, int e, double& p_out,
                     double& rew) {
   double a = act_in(io, c.act_off, e);
   if (c.flags & PGW_F_RESCALE) a = to_raw(a, 0.0, 1.0);
@@ -182,7 +205,8 @@ struct EvTotals {
 // The charging pass shared by the stock station and the Home-Steward charger: window of the
 // event's evaluation time t_now, per-vehicle energy update, charging-set mask, unserved energy
 // of the vehicles that left the window.
-PGW_HD EvTotals ev_charge_pass(const pgw_component& c, const AgentIO& io, int e, double kwh) {
+template <class IO>
+PGW_HD EvTotals ev_charge_pass(const pgw_component& c, const IO& io, int e, double kwh) {
   const double* dp = io.dpar + c.dpar_off;
   const int32_t* ip = io.ipar + c.ipar_off;
   const int words = ip[1], cap = ip[2];
@@ -247,7 +271,8 @@ PGW_HD EvTotals ev_charge_pass(const pgw_component& c, const AgentIO& io, int e,
 // randomised station samples its own vehicles, ev_charging_env.py:154-157): slot i of env e parks
 // from floor(start) to floor(end) minutes, packed into the env's window word i; "parked at t" is
 // evaluated per env (:186-190), the departed vehicles are old charging set \ new one (:194).
-PGW_HD EvTotals ev_charge_pass_env(const pgw_component& c, const AgentIO& io, int e, double kwh) {
+template <class IO>
+PGW_HD EvTotals ev_charge_pass_env(const pgw_component& c, const IO& io, int e, double kwh) {
   const double* dp = io.dpar + c.dpar_off;
   const int32_t* ip = io.ipar + c.ipar_off;
   const int n = ip[0], words = ip[1];
@@ -313,8 +338,8 @@ PGW_HD EvTotals ev_charge_pass_env(const pgw_component& c, const AgentIO& io, in
 // EVENV: the kernel variant that carries the per-env roster path.  It lives in an instantiation of
 // its own (like the Home-Steward house): inlined into the common kernel its register pressure cost
 // every scenario 15-30 % of the component kernel (C3: 61.5 -> 80.2 us, measured).
-template <bool EVENV>
-PGW_HD void ev_advance(const pgw_component& c, const AgentIO& io, int e, double kwh,
+template <bool EVENV, class IO>
+PGW_HD void ev_advance(const pgw_component& c, const IO& io, int e, double kwh,
                        double& p_out, double& rew) {
   const double* dp = io.dpar + c.dpar_off;
   const double mult = dp[2];
@@ -336,14 +361,14 @@ PGW_HD void ev_advance(const pgw_component& c, const AgentIO& io, int e, double 
 #pragma unroll
   for (int j = 0; j < 6; ++j)
     io.obs[(size_t)(c.obs_off + j) * io.E + e] =
-        rs ? to_scaled(raw[j], 0.0, obs_high[j], inv_high[j]) : raw[j];
+        obs_val(io, rs ? to_scaled(raw[j], 0.0, obs_high[j], inv_high[j]) : raw[j]);
   p_out = s_consumed;                                 // kWh per step reported as kW (:255)
   const double over = fmax(0.0, s_consumed - dp[5]);  // :135-142
   rew = div_by(-dp[3] * (unserved * unserved) + -dp[4] * (over * over), dp[6], dp[19]);
 }
 
-template <bool EVENV = false>
-PGW_HD void ev_step(const pgw_component& c, const AgentIO& io, int e, double& p_out,
+template <bool EVENV = false, class IO>
+PGW_HD void ev_step(const pgw_component& c, const IO& io, int e, double& p_out,
                     double& rew) {
   const double* dp = io.dpar + c.dpar_off;
   double a = act_in(io, c.act_off, e);
@@ -351,8 +376,8 @@ PGW_HD void ev_step(const pgw_component& c, const AgentIO& io, int e, double& p_
   ev_advance<EVENV>(c, io, e, (a * dp[0]) * dp[1], p_out, rew);      // :182-183
 }
 
-template <bool EVENV = false>
-PGW_HD void ev_reset(const pgw_component& c, const AgentIO& io, int e) {
+template <bool EVENV = false, class IO>
+PGW_HD void ev_reset(const pgw_component& c, const IO& io, int e) {
   const double* dp = io.dpar + c.dpar_off;
   const int n = io.ipar[c.ipar_off];
   if (EVENV && (c.flags & PGW_F_EV_PER_ENV)) {
@@ -386,7 +411,8 @@ struct BuildingPar {
   const int32_t *u_kind, *u_arg, *obs_src;
 };
 
-PGW_HD BuildingPar building_par(const pgw_component& c, const AgentIO& io) {
+template <class IO>
+PGW_HD BuildingPar building_par(const pgw_component& c, const IO& io) {
   const double* dp = io.dpar + c.dpar_off;
   const int32_t* ip = io.ipar + c.ipar_off;
   BuildingPar b;
@@ -437,7 +463,8 @@ PGW_HD double building_reward(const BuildingPar& b, const Scratch& scr, int t_of
 
 // get_obs (five_zone_rom_env.py:228-283): the 24 possible sources in state-dict order, then
 // the selected ones (obs_src, in that same order) against the bounds in label order.
-PGW_HD void building_obs(const pgw_component& c, const BuildingPar& b, const AgentIO& io,
+template <class IO>
+PGW_HD void building_obs(const pgw_component& c, const BuildingPar& b, const IO& io,
                          int e, const Scratch& scr, double lb, double ub, double t_oa,
                          double p_consumed, double tod, bool grid) {
   PGW_NO_UNROLL
@@ -464,11 +491,12 @@ PGW_HD void building_obs(const pgw_component& c, const BuildingPar& b, const Age
     const double lo = b.low[slot], hi = b.high[slot];
     double o = clip(scr[BSCR_SRC + b.obs_src[slot]], lo, hi);   // np.clip; to_scaled's own clip
     if (rs) o = div_by(2.0 * o - (lo + hi), hi - lo, b.inv[slot]);   // is then the identity
-    io.obs[(size_t)(c.obs_off + slot) * io.E + e] = o;
+    io.obs[(size_t)(c.obs_off + slot) * io.E + e] = obs_val(io, o);
   }
 }
 
-PGW_HD void building_reset(const pgw_component& c, const AgentIO& io, int e) {
+template <class IO>
+PGW_HD void building_reset(const pgw_component& c, const IO& io, int e) {
   const BuildingPar b = building_par(c, io);
   const Scratch& scr = io.scr;
   const double* row = io.drow + c.dtab_off;
@@ -495,7 +523,8 @@ PGW_HD void building_reset(const pgw_component& c, const AgentIO& io, int e) {
                (c.flags & PGW_F_GRID_AWARE) != 0);
 }
 
-PGW_HD void building_step(const pgw_component& c, const AgentIO& io, int e, double& p_out,
+template <class IO>
+PGW_HD void building_step(const pgw_component& c, const IO& io, int e, double& p_out,
                           double& rew) {
   const BuildingPar b = building_par(c, io);
   const Scratch& scr = io.scr;
@@ -552,7 +581,8 @@ PGW_HD double pick5(const double T[5], int i) {
   return v;
 }
 
-PGW_HD void building_step_fast(const pgw_component& c, const AgentIO& io, int e, double& p_out,
+template <class IO>
+PGW_HD void building_step_fast(const pgw_component& c, const IO& io, int e, double& p_out,
                                double& rew) {
   const double* dp = io.dpar + c.dpar_off;
   const int32_t* u_arg = io.ipar + c.ipar_off + 20;
@@ -593,16 +623,16 @@ PGW_HD void building_step_fast(const pgw_component& c, const AgentIO& io, int e,
   sp[5 * E] = p;
 
   const double lb = row[12], ub = row[13];
-  double* op = io.obs + (size_t)c.obs_off * E + e;
+  auto* op = io.obs + (size_t)c.obs_off * E + e;
   double comfort = 0.0;
 #pragma unroll
   for (int z = 0; z < 5; ++z) {
     const double up = Tn[z] - ub, lo = lb - Tn[z];
     double o = clip(up, low[z], high[z]);
-    op[z * E] = rs ? div_by(2.0 * o - (low[z] + high[z]), high[z] - low[z], inv[z]) : o;
+    op[z * E] = obs_val(io, rs ? div_by(2.0 * o - (low[z] + high[z]), high[z] - low[z], inv[z]) : o);
     o = clip(lo, low[5 + z], high[5 + z]);
-    op[(5 + z) * E] =
-        rs ? div_by(2.0 * o - (low[5 + z] + high[5 + z]), high[5 + z] - low[5 + z], inv[5 + z]) : o;
+    op[(5 + z) * E] = obs_val(
+        io, rs ? div_by(2.0 * o - (low[5 + z] + high[5 + z]), high[5 + z] - low[5 + z], inv[5 + z]) : o);
     const double err = fmax(fmax(up, lo), 0.0);
     comfort += err * err;
   }
@@ -611,7 +641,7 @@ PGW_HD void building_step_fast(const pgw_component& c, const AgentIO& io, int e,
   for (int j = 0; j < 5; ++j) {
     const int s = 10 + j;
     const double o = clip(tail[j], low[s], high[s]);
-    op[s * E] = rs ? div_by(2.0 * o - (low[s] + high[s]), high[s] - low[s], inv[s]) : o;
+    op[s * E] = obs_val(io, rs ? div_by(2.0 * o - (low[s] + high[s]), high[s] - low[s], inv[s]) : o);
   }
   const double energy = div_by(-p, 12.0, 1.0 / 12.0);
   rew = dp[45] * energy + dp[46] * (-comfort);
@@ -641,8 +671,8 @@ struct HsTel {
   int E;
   PGW_HD void put(int r, double v) const { if (p) p[(size_t)r * E] = v; }
 };
-template <bool TEL>
-PGW_HD HsTel hs_tel(const pgw_component& c, const AgentIO& io, int e, int own_rows) {
+template <bool TEL, class IO>
+PGW_HD HsTel hs_tel(const pgw_component& c, const IO& io, int e, int own_rows) {
   HsTel t;
   t.E = io.E;
   t.p = (TEL && (c.flags & PGW_F_TELEMETRY)) ? io.sd + (size_t)(c.sd_off + own_rows) * io.E + e
@@ -652,7 +682,8 @@ PGW_HD HsTel hs_tel(const pgw_component& c, const AgentIO& io, int e, int own_ro
 
 // HS_BEGIN  dpar: max_grid_power   dtab: grid_cost of the event
 //           state: pv_power, es_power, es_cost, pv_cost, grid_power (5 rows, the meta state)
-PGW_HD void hs_begin(const pgw_component& c, const AgentIO& io, int e, HsMeta& m, bool first_reset) {
+template <class IO>
+PGW_HD void hs_begin(const pgw_component& c, const IO& io, int e, HsMeta& m, bool first_reset) {
   double* sd = io.sd + (size_t)c.sd_off * io.E + e;
   if (first_reset) {                                   // base_hs.py:53-61
     for (int r = 0; r < 5; ++r) sd[(size_t)r * io.E] = 0.0;
@@ -666,7 +697,8 @@ PGW_HD void hs_begin(const pgw_component& c, const AgentIO& io, int e, HsMeta& m
   m.n = 0;
 }
 
-PGW_HD void hs_end(const pgw_component& c, const AgentIO& io, int e, const HsMeta& m, bool store,
+template <class IO>
+PGW_HD void hs_end(const pgw_component& c, const IO& io, int e, const HsMeta& m, bool store,
                    double& r_agent) {
   if (store) {
     double* sd = io.sd + (size_t)c.sd_off * io.E + e;  // c = the HS_BEGIN descriptor
@@ -688,14 +720,14 @@ PGW_HD void hs_end(const pgw_component& c, const AgentIO& io, int e, const HsMet
 }
 
 // HS_PV  dpar: obs_low, obs_high, 1/(high-low)   dtab: scaled profile value of the event
-template <bool TEL>
-PGW_HD void hs_pv_step(const pgw_component& c, const AgentIO& io, int e, HsMeta& m, bool reset,
+template <bool TEL, class IO>
+PGW_HD void hs_pv_step(const pgw_component& c, const IO& io, int e, HsMeta& m, bool reset,
                        double& p_out) {
   const double* dp = io.dpar + c.dpar_off;
   const bool rs = (c.flags & PGW_F_RESCALE) != 0;
   const double data = io.drow[c.dtab_off];
   const double raw = -data;                            // pv_profile_env_hs.py:110
-  io.obs[(size_t)c.obs_off * io.E + e] = rs ? to_scaled(raw, dp[0], dp[1], dp[2]) : raw;
+  io.obs[(size_t)c.obs_off * io.E + e] = obs_val(io, rs ? to_scaled(raw, dp[0], dp[1], dp[2]) : raw);
   if (reset) {
     m.pv_power = -raw;                                 // only the reset chain sees it (:121-124)
     p_out = 0.0;
@@ -716,14 +748,16 @@ PGW_HD void hs_pv_step(const pgw_component& c, const AgentIO& io, int e, HsMeta&
 //                   max_storage_cost, 1/(hi-lo), 1/max_storage_cost, 1/eta_d, 1/dt, 1/eta_c
 //             ipar: storage ordinal
 //             state: SOC, current_cost
-PGW_HD void hs_storage_obs(const pgw_component& c, const AgentIO& io, int e, double soc, double cost) {
+template <class IO>
+PGW_HD void hs_storage_obs(const pgw_component& c, const IO& io, int e, double soc, double cost) {
   const double* dp = io.dpar + c.dpar_off;
   const bool rs = (c.flags & PGW_F_RESCALE) != 0;
-  io.obs[(size_t)c.obs_off * io.E + e] = rs ? to_scaled(soc, dp[0], dp[1], dp[9]) : soc;
-  io.obs[(size_t)(c.obs_off + 1) * io.E + e] = rs ? to_scaled(cost, 0.0, dp[8], dp[10]) : cost;
+  io.obs[(size_t)c.obs_off * io.E + e] = obs_val(io, rs ? to_scaled(soc, dp[0], dp[1], dp[9]) : soc);
+  io.obs[(size_t)(c.obs_off + 1) * io.E + e] = obs_val(io, rs ? to_scaled(cost, 0.0, dp[8], dp[10]) : cost);
 }
 
-PGW_HD void hs_storage_reset(const pgw_component& c, const AgentIO& io, int e, bool first_reset) {
+template <class IO>
+PGW_HD void hs_storage_reset(const pgw_component& c, const IO& io, int e, bool first_reset) {
   const double* dp = io.dpar + c.dpar_off;
   double* sd = io.sd + (size_t)c.sd_off * io.E + e;
   const int ord = io.ipar[c.ipar_off];
@@ -735,8 +769,8 @@ PGW_HD void hs_storage_reset(const pgw_component& c, const AgentIO& io, int e, b
   hs_storage_obs(c, io, e, soc, sd[(size_t)1 * io.E]);
 }
 
-template <bool TEL>
-PGW_HD void hs_storage_step(const pgw_component& c, const AgentIO& io, int e, HsMeta& m,
+template <bool TEL, class IO>
+PGW_HD void hs_storage_step(const pgw_component& c, const IO& io, int e, HsMeta& m,
                             double& p_out) {
   const double* dp = io.dpar + c.dpar_off;
   const double lo = dp[0], hi = dp[1], eta_c = dp[2], eta_d = dp[3], pmax = dp[4], dt = dp[5];
@@ -806,8 +840,8 @@ PGW_HD void hs_storage_step(const pgw_component& c, const AgentIO& io, int e, Hs
 //              1 / max_charge_cost
 //        dtab: evaluation time, new time      itab: as the stock station
 //        state: n energy rows + current_cost; words of the charging set
-template <bool TEL>
-PGW_HD void hs_ev_advance(const pgw_component& c, const AgentIO& io, int e, double a_raw, HsMeta& m,
+template <bool TEL, class IO>
+PGW_HD void hs_ev_advance(const pgw_component& c, const IO& io, int e, double a_raw, HsMeta& m,
                           bool reset, double& p_out) {
   const double* dp = io.dpar + c.dpar_off;
   const int n = io.ipar[c.ipar_off];
@@ -857,7 +891,7 @@ PGW_HD void hs_ev_advance(const pgw_component& c, const AgentIO& io, int e, doub
   for (int j = 0; j < 7; ++j) {
     const double hi = j < 6 ? obs_high[j] : max_cost;
     const double inv = j < 6 ? dp[13 + j] : dp[23 + 2 * n];
-    io.obs[(size_t)(c.obs_off + j) * io.E + e] = rs ? to_scaled(raw[j], 0.0, hi, inv) : raw[j];
+    io.obs[(size_t)(c.obs_off + j) * io.E + e] = obs_val(io, rs ? to_scaled(raw[j], 0.0, hi, inv) : raw[j]);
   }
   if (!reset) {
     m.pv_power = loc.pv_power; m.es_power = loc.es_power; m.grid_power = loc.grid_power;
@@ -880,8 +914,8 @@ PGW_HD void hs_ev_advance(const pgw_component& c, const AgentIO& io, int e, doub
   p_out = real_power;
 }
 
-template <bool TEL>
-PGW_HD void hs_ev_reset(const pgw_component& c, const AgentIO& io, int e, HsMeta& m) {
+template <bool TEL, class IO>
+PGW_HD void hs_ev_reset(const pgw_component& c, const IO& io, int e, HsMeta& m) {
   const double* dp = io.dpar + c.dpar_off;
   const int n = io.ipar[c.ipar_off];
   const double* e0 = dp + 21 + n;
@@ -894,8 +928,8 @@ PGW_HD void hs_ev_reset(const pgw_component& c, const AgentIO& io, int e, HsMeta
 
 // HS_DEVICES  dpar: minutes_per_step / 60, obs_high[k], 1/obs_high[k]     ipar: k (columns)
 //             dtab: scaled row [k] (observation), unscaled row [k] (demand)
-template <bool TEL>
-PGW_HD void hs_devices_step(const pgw_component& c, const AgentIO& io, int e, HsMeta& m, bool reset,
+template <bool TEL, class IO>
+PGW_HD void hs_devices_step(const pgw_component& c, const IO& io, int e, HsMeta& m, bool reset,
                             double& p_out) {
   const double* dp = io.dpar + c.dpar_off;
   const int k = io.ipar[c.ipar_off];
@@ -903,7 +937,7 @@ PGW_HD void hs_devices_step(const pgw_component& c, const AgentIO& io, int e, Hs
   const double* row = io.drow + c.dtab_off;
   for (int j = 0; j < k; ++j)
     io.obs[(size_t)(c.obs_off + j) * io.E + e] =
-        rs ? to_scaled(row[j], 0.0, dp[1 + j], dp[1 + k + j]) : row[j];
+        obs_val(io, rs ? to_scaled(row[j], 0.0, dp[1 + j], dp[1 + k + j]) : row[j]);
   p_out = 0.0;
   if (reset) return;
   double a = act_in(io, c.act_off, e);
@@ -943,8 +977,8 @@ PGW_HD bool is_house(const pgw_agent& ag, const pgw_component* comps) {
 
 // Home-Steward house (base_hs.py:120-178).  Kept apart from agent_step so that kernels of
 // scenarios without a house do not carry its code and stack frame.
-template <bool TEL>
-PGW_HD void house_step(const pgw_agent& ag, const pgw_component* comps, const AgentIO& io, int e,
+template <bool TEL, class IO>
+PGW_HD void house_step(const pgw_agent& ag, const pgw_component* comps, const IO& io, int e,
                        double& p_agent, double& r_agent) {
   p_agent = 0.0;
   HsMeta m;
@@ -970,8 +1004,8 @@ PGW_HD void house_step(const pgw_agent& ag, const pgw_component* comps, const Ag
 }
 
 // base_hs.py:67-92; the meta state itself is not reset
-template <bool TEL>
-PGW_HD void house_reset(const pgw_agent& ag, const pgw_component* comps, const AgentIO& io, int e,
+template <bool TEL, class IO>
+PGW_HD void house_reset(const pgw_agent& ag, const pgw_component* comps, const IO& io, int e,
                         bool first_reset) {
   HsMeta m;
   hs_begin(comps[ag.comp_begin], io, e, m, first_reset);
@@ -988,8 +1022,8 @@ PGW_HD void house_reset(const pgw_agent& ag, const pgw_component* comps, const A
   }
 }
 
-template <bool EVENV = false>
-PGW_HD void agent_step(const pgw_agent& ag, const pgw_component* comps, const AgentIO& io, int e,
+template <bool EVENV = false, class IO>
+PGW_HD void agent_step(const pgw_agent& ag, const pgw_component* comps, const IO& io, int e,
                        double& p_agent, double& r_agent) {
   p_agent = 0.0;
   r_agent = 0.0;
@@ -1011,8 +1045,8 @@ PGW_HD void agent_step(const pgw_agent& ag, const pgw_component* comps, const Ag
   }
 }
 
-template <bool EVENV = false>
-PGW_HD void agent_reset(const pgw_agent& ag, const pgw_component* comps, const AgentIO& io, int e) {
+template <bool EVENV = false, class IO>
+PGW_HD void agent_reset(const pgw_agent& ag, const pgw_component* comps, const IO& io, int e) {
   for (int ci = ag.comp_begin; ci < ag.comp_end; ++ci) {
     const pgw_component c = comps[ci];
     switch (c.type) {

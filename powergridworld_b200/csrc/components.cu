@@ -12,6 +12,8 @@
 //
 // Replaces HOT LOOP 1-3 of gridworld/multiagent_env.py:165-181 and gridworld/base.py:125-137.
 // Compiled with -fmad=false (see component_math.cuh).
+#include <type_traits>
+
 #include "component_math.cuh"
 #include "internal.cuh"
 #include "tma.cuh"
@@ -21,8 +23,10 @@ namespace pgw {
 // HOUSE: the scenario contains Home-Steward houses (their code stays out of the other kernel);
 // TEL: some of their components record step_meta telemetry.
 // EVENV: some charging station runs on per-env rosters (PGW_F_EV_PER_ENV).
-template <bool HOUSE, bool TEL, bool EVENV = false>
+// IO32: the caller's actions and observations are float arrays (p.io32), else double.
+template <bool HOUSE, bool TEL, bool EVENV = false, bool IO32 = false>
 __global__ void __launch_bounds__(64, 10) component_kernel(const CompParams p) {
+  using IoT = typename std::conditional<IO32, float, double>::type;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ __align__(8) uint64_t mbar[2];
   // [comps slice | dpar slice | ipar slice | double event row | int event row | scratch]
@@ -89,14 +93,14 @@ __global__ void __launch_bounds__(64, 10) component_kernel(const CompParams p) {
   const int event = ev;
   const pgw_component* comps = s_comps - sl.c_lo;      // indexed by absolute component number
 
-  AgentIO io;
+  AgentIOT<IoT, IoT> io;
   io.scr.p = scratch + threadIdx.x;          // [kScratchDoubles][blockDim.x]: conflict-free
   io.scr.stride = blockDim.x;
   io.E = p.E;
-  io.actions = p.actions;
+  io.actions = static_cast<const IoT*>(p.actions);
   io.aE = p.E;
   io.ae0 = 0;
-  io.obs = p.obs;
+  io.obs = static_cast<IoT*>(p.obs);
   io.sd = p.sd;
   io.si = p.si;
   io.init_soc = p.init_soc;
@@ -119,7 +123,8 @@ __global__ void __launch_bounds__(64, 10) component_kernel(const CompParams p) {
         const pgw_component c = comps[ci];
         const int na = c.type == PGW_BUILDING ? 6 : 1;
         for (int r = 0; r < na; ++r)
-          asm volatile("prefetch.global.L1 [%0];" ::"l"(p.actions + (size_t)(c.act_off + r) * p.E + e));
+          asm volatile("prefetch.global.L1 [%0];"
+                       ::"l"(static_cast<const IoT*>(p.actions) + (size_t)(c.act_off + r) * p.E + e));
         const int ns = c.type == PGW_BUILDING ? 6 : (c.type == PGW_STORAGE ? 1 : 0);
         for (int r = 0; r < ns; ++r)
           asm volatile("prefetch.global.L1 [%0];" ::"l"(p.sd + (size_t)(c.sd_off + r) * p.E + e));
@@ -162,20 +167,35 @@ __global__ void __launch_bounds__(64, 10) component_kernel(const CompParams p) {
 #endif
 }
 
+template <bool IO32>
+static bool is_component_kernel_io(const void* func) {
+  return func == (const void*)component_kernel<false, false, false, IO32> ||
+         func == (const void*)component_kernel<true, false, false, IO32> ||
+         func == (const void*)component_kernel<true, true, false, IO32> ||
+         func == (const void*)component_kernel<false, false, true, IO32> ||
+         func == (const void*)component_kernel<true, false, true, IO32> ||
+         func == (const void*)component_kernel<true, true, true, IO32>;
+}
+
 bool is_component_kernel(const void* func) {
-  return func == (const void*)component_kernel<false, false> || func == (const void*)component_kernel<true, false> ||
-         func == (const void*)component_kernel<true, true> || func == (const void*)component_kernel<false, false, true> ||
-         func == (const void*)component_kernel<true, false, true> || func == (const void*)component_kernel<true, true, true>;
+  return is_component_kernel_io<false>(func) || is_component_kernel_io<true>(func);
+}
+
+template <bool IO32>
+static auto component_kernel_for(const CompParams& p) {
+  if (p.ev_per_env)
+    return p.has_house ? (p.has_house > 1 ? component_kernel<true, true, true, IO32>
+                                          : component_kernel<true, false, true, IO32>)
+                       : component_kernel<false, false, true, IO32>;
+  return p.has_house ? (p.has_house > 1 ? component_kernel<true, true, false, IO32>
+                                        : component_kernel<true, false, false, IO32>)
+                     : component_kernel<false, false, false, IO32>;
 }
 
 cudaError_t launch_components(const CompParams& p, int smem_bytes, cudaStream_t s) {
   const int threads = 64;      // small CTAs: a 4096-env batch still reaches every SM
   dim3 grid(p.num_ctas);       // the CTA -> (agent, env blocks) table is built in pgw_create
-  auto kern = p.has_house ? (p.has_house > 1 ? component_kernel<true, true> : component_kernel<true, false>)
-                          : component_kernel<false, false>;
-  if (p.ev_per_env)
-    kern = p.has_house ? (p.has_house > 1 ? component_kernel<true, true, true> : component_kernel<true, false, true>)
-                       : component_kernel<false, false, true>;
+  auto kern = p.io32 ? component_kernel_for<true>(p) : component_kernel_for<false>(p);
   if (smem_bytes > 48 * 1024) {
     cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes);
     if (err != cudaSuccess) return err;

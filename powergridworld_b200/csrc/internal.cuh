@@ -33,6 +33,7 @@ struct CompParams {
   int advance_clock;       // 1 when this kernel is the last one of the step (no feeder)
   int clip_init_soc;       // reset: clip init_soc to each storage's range (PGW_OPT_CLIP_INIT_SOC)
   int pdl_trigger;         // griddepcontrol.launch_dependents: 0 never, 1 after the clock read, 2 at the end
+  int io32;                // 1: actions and obs are float arrays (the IO32 kernel instantiations), 0: double
   long long* phase_clk;    // PGW_PHASE_TIMERS builds only: [CTA][8] globaltimer at entry / exit + SM-clock stamps
   int owns_reward;         // 1 when no later kernel changes the reward (no feeder / no penalty)
   int has_house;           // 1: the scenario contains Home-Steward houses, 2: with telemetry
@@ -49,8 +50,8 @@ struct CompParams {
   const double* dtab;
   const int32_t* itab;
   int dstride, istride;
-  const double* actions;
-  double* obs;
+  const void* actions;      // [act_dim][E] double, or float under io32
+  void* obs;               // [obs_dim][E] double, or float under io32
   double* rew;
   double* rew_copy;        // internal copy of the step's rewards (pgw_stats), written when this
                            // kernel owns the final reward (no feeder)

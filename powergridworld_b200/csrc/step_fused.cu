@@ -34,6 +34,8 @@
 //
 // Compiled -fmad=false like components.cu (the component arithmetic must round like NumPy);
 // the power-flow code spells out its fused multiply-adds.
+#include <type_traits>
+
 #include "component_math.cuh"
 #include "internal.cuh"
 #include "tc2_common.cuh"
@@ -91,9 +93,11 @@ __host__ __device__ inline SfLayout sf_layout(const FusedParams& P) {
 #define SF_STAMP(k) do { } while (0)
 #endif
 
-template <bool ANY_M5>
+// IO32: the caller's actions and observations are float arrays (P.c.io32), else double.
+template <bool ANY_M5, bool IO32 = false>
 __global__ void __launch_bounds__(SF_THREADS, 1)
     step_fused_kernel(const __grid_constant__ FusedParams P) {
+  using IoT = typename std::conditional<IO32, float, double>::type;
   extern __shared__ __align__(1024) unsigned char sf_smem[];
   __shared__ __align__(8) uint64_t mbar_tab, mbar_ev, mbar_act;
   const CompParams& pc = P.c;
@@ -124,7 +128,7 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   double* sVn = reinterpret_cast<double*>(sf_smem + L.vn);         // [16][env]
   double* sCp = reinterpret_cast<double*>(sf_smem + L.cp);         // [C][env]
   double* sCr = reinterpret_cast<double*>(sf_smem + L.cr);
-  double* sAct = reinterpret_cast<double*>(sf_smem + L.act);
+  IoT* sAct = reinterpret_cast<IoT*>(sf_smem + L.act);
 
   // ---- prologue: clock, staging of everything that is shared by the envs
   bool first_tile = true;
@@ -167,24 +171,30 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   const int span = P.e_hi - P.e_lo;
   const int tiles = (span + SF_ENVS - 1) / SF_ENVS;
   // The actions of a (full) tile are fetched into shared memory by TMA bulk copies, one 256-byte
-  // row segment each, issued by warp 1 at kernel entry / while the previous tile's power flow
+  // (float: 128-byte) row segment each, issued by warp 1 at kernel entry / while the previous tile's power flow
   // runs: the component steps then find them on chip.  (The first fetch used to be issued after
   // the tables had landed: a second ~1.4 us TMA round trip in front of the component steps.)
   // With actions in HOST memory this is what decouples the PCIe reads from the component code, and
   // CTA b delays its first fetch by b x stagger_cycles so that the link serves the tiles in order
   // -- the first tiles write their observations (GPU -> host) while the last ones still wait for
   // their actions (host -> GPU).
+  // (a bulk copy needs a 16-byte aligned source: every row segment of the tile must start on one.  A float32
+  // caller's array may start 4 or 8 bytes past a 16-byte boundary, e.g. a view into a larger tensor: its
+  // tiles then read their actions from global memory)
+  constexpr int kAlign = 16 / (int)sizeof(IoT);
+  const bool act_aligned = !IO32 || (reinterpret_cast<uintptr_t>(pc.actions) & 15u) == 0;
   auto tile_in_smem = [&](int tile) {
     const int e0 = P.e_lo + tile * SF_ENVS;
-    return (E % 2 == 0) && (e0 % 2 == 0) && e0 + SF_ENVS <= P.e_hi;
+    return act_aligned && (E % kAlign == 0) && (e0 % kAlign == 0) && e0 + SF_ENVS <= P.e_hi;
   };
   auto fetch_actions = [&](int tile) {                 // warp 1
     if (tile < tiles && tile_in_smem(tile)) {
       const int e0 = P.e_lo + tile * SF_ENVS;
-      if (lane == 0) mbar_expect_tx(&mbar_act, (uint32_t)P.act_dim * SF_ENVS * 8u);
+      if (lane == 0) mbar_expect_tx(&mbar_act, (uint32_t)P.act_dim * SF_ENVS * (uint32_t)sizeof(IoT));
       __syncwarp();
       for (int r = lane; r < P.act_dim; r += 32)
-        tma_bulk_g2s(sAct + (size_t)r * SF_ENVS, pc.actions + (size_t)r * E + e0, SF_ENVS * 8u, &mbar_act);
+        tma_bulk_g2s(sAct + (size_t)r * SF_ENVS, static_cast<const IoT*>(pc.actions) + (size_t)r * E + e0,
+                     SF_ENVS * (uint32_t)sizeof(IoT), &mbar_act);
     }
   };
   if (w == 1) {
@@ -231,14 +241,14 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   const int32_t* lidx = reinterpret_cast<const int32_t*>(sT + t.t_lidx);
   const int32_t* anode = reinterpret_cast<const int32_t*>(sT + t.t_anode);
 
-  AgentIO io;
+  AgentIOT<IoT, IoT> io;
   io.scr.p = nullptr;                                  // table-driven building path: not in this kernel
   io.scr.stride = 0;
   io.E = E;
-  io.actions = pc.actions;
+  io.actions = static_cast<const IoT*>(pc.actions);
   io.aE = E;
   io.ae0 = 0;
-  io.obs = pc.obs;
+  io.obs = static_cast<IoT*>(pc.obs);
   io.sd = pc.sd;
   io.si = pc.si;
   io.init_soc = nullptr;
@@ -291,7 +301,7 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
       act_phase ^= 1u;
       io.actions = sAct; io.aE = SF_ENVS; io.ae0 = P.e_lo + tile * SF_ENVS;
     } else {
-      io.actions = pc.actions; io.aE = E; io.ae0 = 0;
+      io.actions = static_cast<const IoT*>(pc.actions); io.aE = E; io.ae0 = 0;
     }
     SF_STAMP(3);
 
@@ -560,7 +570,8 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
 }
 
 bool is_step_fused_kernel(const void* func) {
-  return func == (const void*)step_fused_kernel<false> || func == (const void*)step_fused_kernel<true>;
+  return func == (const void*)step_fused_kernel<false, false> || func == (const void*)step_fused_kernel<true, false> ||
+         func == (const void*)step_fused_kernel<false, true> || func == (const void*)step_fused_kernel<true, true>;
 }
 
 size_t step_fused_smem_bytes(const FusedParams& P) { return sf_layout(P).total; }
@@ -568,7 +579,8 @@ size_t step_fused_smem_bytes(const FusedParams& P) { return sf_layout(P).total; 
 int step_fused_tiles(int envs) { return (envs + SF_ENVS - 1) / SF_ENVS; }
 
 cudaError_t launch_step_fused(const FusedParams& P, int grid, cudaStream_t s, bool programmatic) {
-  auto kern = P.f.tc2.any_m5 ? step_fused_kernel<true> : step_fused_kernel<false>;
+  auto kern = P.c.io32 ? (P.f.tc2.any_m5 ? step_fused_kernel<true, true> : step_fused_kernel<false, true>)
+                       : (P.f.tc2.any_m5 ? step_fused_kernel<true, false> : step_fused_kernel<false, false>);
   const size_t smem = step_fused_smem_bytes(P);
   cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (err != cudaSuccess) return err;

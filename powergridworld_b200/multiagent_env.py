@@ -13,6 +13,12 @@ handle.  ``reset``/``step`` then run entirely on the GPU:
     ``[rows, num_envs]`` (env index fastest), and ``step_host`` / ``reset_host`` on
     pinned host arrays (the end-to-end path).
 
+``io_dtype="float32"`` makes the actions and observations of the batched and host-buffer
+calls float32 (the dtype of a policy network's inputs and outputs).  The simulation itself
+stays float64: actions are widened where the kernels read them, observations are computed
+in float64 and rounded to nearest when stored.  Rewards, done flags, initial SOCs and all
+state keep their types.  The dict API keeps the reference's float64 contract.
+
 Deviations from the reference, all deliberate: ``history`` is only recorded when
 ``record_history=True``; overriding ``get_external_obs_vars`` is rejected (the grid
 variables are assembled on the device with the reference's one-step lag).  The
@@ -148,7 +154,7 @@ class MultiAgentEnv(_Env):
                  max_episode_steps: int = None, rescale_spaces: bool = True,
                  num_envs: int = 1, device=None, record_history: bool = False,
                  pf_tol: float = None, pf_max_iter: int = None, pf_kernel: str = "fp64",
-                 _dry_run: bool = False, **kwargs):
+                 io_dtype: str = "float64", _dry_run: bool = False, **kwargs):
         if type(self).get_external_obs_vars is not MultiAgentEnv.get_external_obs_vars:
             raise NotImplementedError(
                 "overriding get_external_obs_vars is not supported: grid variables are "
@@ -164,6 +170,9 @@ class MultiAgentEnv(_Env):
         self.pf_config = pf_config
         self.max_episode_steps = max_episode_steps if max_episode_steps is not None else np.inf
         self.num_envs = int(num_envs)
+        if io_dtype not in self._IO_DTYPES:
+            raise ValueError(f"io_dtype must be one of {list(self._IO_DTYPES)}, not {io_dtype!r}")
+        self.io_dtype = io_dtype
         self.record_history = record_history
         self.episode_step = None
         self.history = None
@@ -213,6 +222,8 @@ class MultiAgentEnv(_Env):
     # the oracle to ~1e-9 p.u.), "tc" / "tc2" = tcgen05 solvers (1e-6 p.u., what bench.py runs),
     # "auto" = tc2 when the feeder fits it (<= 88 load branches), else fp64
     _PF_KERNELS = {"fp64": 0, "tc": 1, "tc2": 2, "auto": 2}
+    # element type of the actions / observations of the batched and host-buffer API
+    _IO_DTYPES = ("float64", "float32")
 
     def _select_pf_kernel(self, name: str):
         try:
@@ -381,10 +392,17 @@ class MultiAgentEnv(_Env):
         self._lib = lib
         E, A = self.num_envs, len(self.agents)
         f64 = dict(dtype=torch.float64, device=self.device)
-        self.obs = torch.zeros((self.obs_dim, E), **f64)
+        io32 = self.io_dtype == "float32"
+        self._io_torch = torch.float32 if io32 else torch.float64
+        self._pgw_reset = lib.pgw_reset_f32 if io32 else lib.pgw_reset
+        self._pgw_step = lib.pgw_step_f32 if io32 else lib.pgw_step
+        self._pgw_reset_host = lib.pgw_reset_host_f32 if io32 else lib.pgw_reset_host
+        self._pgw_step_host = lib.pgw_step_host_f32 if io32 else lib.pgw_step_host
+        io = dict(dtype=self._io_torch, device=self.device)
+        self.obs = torch.zeros((self.obs_dim, E), **io)
         self.rew = torch.zeros((A, E), **f64)
         self.done = torch.zeros((E,), dtype=torch.uint8, device=self.device)
-        self._act = torch.zeros((self.act_dim, E), **f64)
+        self._act = torch.zeros((self.act_dim, E), **io)
         self._act_shape = self._act.shape
         self._obs_ptr, self._rew_ptr = self.obs.data_ptr(), self.rew.data_ptr()
         self._done_ptr = self.done.data_ptr()
@@ -533,8 +551,7 @@ class MultiAgentEnv(_Env):
             self._soc = soc
             soc_ptr = C.c_void_p(soc.data_ptr())
         with torch.cuda.device(self.device):
-            N.check(self._lib.pgw_reset(self._h, soc_ptr, C.c_void_p(self.obs.data_ptr()),
-                                        self._stream()))
+            N.check(self._pgw_reset(self._h, soc_ptr, C.c_void_p(self.obs.data_ptr()), self._stream()))
         self.episode_step = 0
         self._needs_reset = False
         self._lag = None
@@ -543,23 +560,23 @@ class MultiAgentEnv(_Env):
         return self.obs
 
     def step_batch(self, actions):
-        """actions ``[act_dim, E]`` float64 device tensor -> (obs, rew, done, all_done).
-        The returned tensors are the env's own buffers, overwritten by the next call."""
+        """actions ``[act_dim, E]`` device tensor of the env's ``io_dtype`` -> (obs, rew, done,
+        all_done).  The returned tensors are the env's own buffers, overwritten by the next call."""
         torch = _torch()
         if self._needs_reset:
             raise RuntimeError("call reset before step")
-        if actions.dtype != torch.float64 or actions.shape != self._act_shape \
+        if actions.dtype != self._io_torch or actions.shape != self._act_shape \
                 or not actions.is_contiguous() or actions.device != self.device:
-            raise ValueError(f"actions must be a contiguous float64 [{self.act_dim}, "
+            raise ValueError(f"actions must be a contiguous {self.io_dtype} [{self.act_dim}, "
                              f"{self.num_envs}] tensor on {self.device}")
         stream = torch.cuda.current_stream(self.device).cuda_stream
         if torch.cuda.current_device() == self._dev_index:
-            rc = self._lib.pgw_step(self._h, actions.data_ptr(), self._obs_ptr, self._rew_ptr,
-                                    self._done_ptr, stream)
+            rc = self._pgw_step(self._h, actions.data_ptr(), self._obs_ptr, self._rew_ptr,
+                                self._done_ptr, stream)
         else:                                       # the caller's current device is another GPU
             with torch.cuda.device(self.device):
-                rc = self._lib.pgw_step(self._h, actions.data_ptr(), self._obs_ptr, self._rew_ptr,
-                                        self._done_ptr, stream)
+                rc = self._pgw_step(self._h, actions.data_ptr(), self._obs_ptr, self._rew_ptr,
+                                    self._done_ptr, stream)
         if rc:
             N.check(rc)
         self.episode_step += 1
@@ -574,7 +591,8 @@ class MultiAgentEnv(_Env):
             torch = _torch()
             E, A = self.num_envs, len(self.agents)
             mk = lambda *s, dt=torch.float64: torch.zeros(s, dtype=dt).pin_memory()
-            self._pin = dict(act=mk(self.act_dim, E), obs=mk(self.obs_dim, E), rew=mk(A, E),
+            io = self._io_torch
+            self._pin = dict(act=mk(self.act_dim, E, dt=io), obs=mk(self.obs_dim, E, dt=io), rew=mk(A, E),
                              done=mk(E, dt=torch.uint8), soc=mk(max(self.num_storage, 1), E))
         return self._pin
 
@@ -587,15 +605,17 @@ class MultiAgentEnv(_Env):
             pin["soc"][:self.num_storage].copy_(torch.as_tensor(np.asarray(init_storage, dtype=np.float64)))
             soc_ptr = C.c_void_p(pin["soc"].data_ptr())
         with torch.cuda.device(self.device):
-            N.check(self._lib.pgw_reset_host(self._h, soc_ptr, C.c_void_p(pin["obs"].data_ptr()),
-                                             self._stream()))
+            N.check(self._pgw_reset_host(self._h, soc_ptr, C.c_void_p(pin["obs"].data_ptr()),
+                                         self._stream()))
         self.episode_step = 0
         self._needs_reset = False
         return pin["obs"].numpy()
 
     def step_host(self, actions: np.ndarray):
         """``actions`` host array [act_dim, E] -> (obs, rew, done) host arrays (pinned buffers
-        owned by the env).  Copies to and from the device are part of the call."""
+        owned by the env; obs in the env's ``io_dtype``).  Copies to and from the device are part
+        of the call; actions that are not a page-locked array of the env's dtype are copied into
+        the env's pinned action buffer first."""
         torch = _torch()
         if self._needs_reset:
             raise RuntimeError("call reset before step")
@@ -611,11 +631,11 @@ class MultiAgentEnv(_Env):
         if isinstance(actions, torch.Tensor):
             src = actions
         else:
-            src = torch.from_numpy(np.ascontiguousarray(actions, dtype=np.float64))
+            src = torch.from_numpy(np.ascontiguousarray(actions, dtype=self.io_dtype))
         if src.numel() != hs["numel"]:
             raise ValueError(f"actions must be [{self.act_dim}, {self.num_envs}]")
         act_ptr = src.data_ptr()
-        ok = src.dtype == torch.float64 and src.is_contiguous()
+        ok = src.dtype == self._io_torch and src.is_contiguous()
         if ok:                                      # page-locked as well: the DMA reads it in place
             ok = hs["pinned"].get(act_ptr)          # (is_pinned() is a driver query: remembered)
             if ok is None:
@@ -628,10 +648,10 @@ class MultiAgentEnv(_Env):
         po, pr, pd = hs["ptrs"]
         stream = torch.cuda.current_stream(self.device).cuda_stream
         if torch.cuda.current_device() == hs["dev"]:
-            rc = self._lib.pgw_step_host(self._h, act_ptr, po, pr, pd, stream)
+            rc = self._pgw_step_host(self._h, act_ptr, po, pr, pd, stream)
         else:
             with torch.cuda.device(self.device):
-                rc = self._lib.pgw_step_host(self._h, act_ptr, po, pr, pd, stream)
+                rc = self._pgw_step_host(self._h, act_ptr, po, pr, pd, stream)
         if rc:
             N.check(rc)
         self.episode_step += 1
@@ -673,7 +693,8 @@ class MultiAgentEnv(_Env):
                      N.FIELD_EP_RETURN, N.FIELD_PF_STATE)
 
     def state_dict(self) -> dict:
-        """Everything needed to resume the batch bit for bit: device fields + episode clock."""
+        """Everything needed to resume the batch bit for bit: device fields + episode clock (the
+        last observations in the env's ``io_dtype``)."""
         fields = {}
         for f in self._STATE_FIELDS:
             if self.pf_solver is None and f in (N.FIELD_VOLTAGES, N.FIELD_VMIN, N.FIELD_VMAX,
@@ -693,6 +714,9 @@ class MultiAgentEnv(_Env):
 
     def load_state_dict(self, state: dict):
         torch = _torch()
+        if state["obs"].dtype != self.obs.dtype:
+            raise ValueError(f"checkpoint observations are {state['obs'].dtype}, this env's io_dtype is "
+                             f"{self.io_dtype}: load it into an env with the io_dtype it was taken with")
         rand = self._randomised()
         if rand:
             rosters = state.get("rosters")
@@ -775,6 +799,13 @@ class MultiAgentEnv(_Env):
         if self.num_envs != 1:
             raise RuntimeError("the dict API serves num_envs == 1; use reset_batch/step_batch")
 
+    def _require_dict_api(self):
+        self._require_single()
+        if self.io_dtype != "float64":
+            raise RuntimeError(f"the dict API keeps the reference's float64 observations and actions; "
+                               f"with io_dtype={self.io_dtype!r} use reset_batch/step_batch or "
+                               "reset_host/step_host")
+
     def _obs_dict(self, flat: np.ndarray) -> dict:
         out = {}
         for ag in self.agents:
@@ -799,7 +830,7 @@ class MultiAgentEnv(_Env):
     def reset(self, init_storage=None) -> Dict[str, any]:
         """multiagent_env.py:125-140.  ``init_storage`` ([num_storage] or [num_storage, 1])
         overrides the host RNG draw of the storages' initial SOC."""
-        self._require_single()
+        self._require_dict_api()
         if init_storage is not None:
             init_storage = np.asarray(init_storage, dtype=np.float64).reshape(self.num_storage, 1)
         obs = self.reset_batch(init_storage)
@@ -838,12 +869,12 @@ class MultiAgentEnv(_Env):
                 for i, a in enumerate(self.agents)}
 
     def get_obs(self) -> Dict[str, any]:
-        self._require_single()
+        self._require_dict_api()
         return self._obs_dict(self.obs[:, 0].cpu().numpy())
 
     def step(self, action: Dict[str, any]):
         """multiagent_env.py:151-212 for the single-env case."""
-        self._require_single()
+        self._require_dict_api()
         torch = _torch()
         self._act.copy_(torch.from_numpy(self.flatten_action(action)).reshape(self.act_dim, 1))
         obs, rew, _, all_done = self.step_batch(self._act)
