@@ -824,16 +824,39 @@ int pgw_create(const pgw_spec* spec, pgw_env** out) {
         t.f_kc = putf(&env->tc2c, sizeof(env->tc2c));
         t.f_kp = putf(&env->tc2p, sizeof(env->tc2p));
         t.f_aslot = putf(aslot.data(), aslot.size() * 4);
-        // Znb^T / xscale of the expansion slots in float32 ([k][slot], 16 ncc slots a row): the
-        // fused kernel's v = w - Znb i on the SIMT pipe, from the fixed point's scaled currents
-        const int nxs = NBP * ncc;
-        std::vector<float2> xz((size_t)NBP * nxs, make_float2(0.f, 0.f));
-        for (int k = 0; k < nb; ++k)
-          for (int sidx = 0; sidx < nx; ++sidx) {
-            const double2 z = ZN(xnode[sidx], k);
-            xz[(size_t)k * nxs + sidx] = make_float2((float)(z.x / xs), (float)(z.y / xs));
-          }
-        t.f_xz = putf(xz.data(), xz.size() * sizeof(float2));
+        // B fragments of the fused kernel's mma.sync.m16n8k16 products: the realified operator
+        // (rows: outputs, columns: the 16 branch currents) x scale, split into FP16 hi / lo as
+        // images() does, with (Re, Im) interleaved per item along N (the outputs) and K (the
+        // currents): n-tile j = outputs 4j .. 4j + 3.  In the order the registers take them:
+        // [n-tile][lane][k-step][hi b0, hi b1, lo b0, lo b1], two 16-byte loads a lane.
+        auto mma_frags = [&](std::vector<uint16_t>& bf, int ntiles, int nitems, double scale, auto&& zget) {
+          const size_t base = bf.size();
+          bf.resize(base + (size_t)ntiles * 32 * 2 * 4 * 2, 0);
+          for (int j = 0; j < ntiles; ++j)
+            for (int lane = 0; lane < 32; ++lane) {
+              const int g = lane >> 2, tq = lane & 3;
+              const int r = 4 * j + g / 2;               // output item of column 8j + g
+              const bool im_out = (g & 1) != 0;
+              for (int s = 0; s < 2; ++s)
+                for (int reg = 0; reg < 2; ++reg)
+                  for (int ii = 0; ii < 2; ++ii) {       // the two halves: Re / Im of current q
+                    const int q = 8 * s + tq + 4 * reg;
+                    const double2 z = (r < nitems && q < nb) ? zget(r, q) : make_double2(0.0, 0.0);
+                    const double v = (im_out ? (ii ? -z.x : -z.y) : (ii ? z.y : -z.x)) * scale;
+                    const __half hi = __float2half_rn((float)v);
+                    const __half lo = __float2half_rn((float)(v - (double)__half2float(hi)));
+                    const size_t o = base + ((((size_t)j * 32 + lane) * 2 + s) * 4 + reg) * 2 + ii;
+                    memcpy(&bf[o], &hi, 2);
+                    memcpy(&bf[o + 4], &lo, 2);
+                  }
+            }
+        };
+        // f_xz: 4 n-tiles of the fixed point's drops (Zbb x sb1), then 4 per chunk of 16 slots of
+        // the expansion's node voltages (Znb of the expansion slots x sb2)
+        std::vector<uint16_t> bf;
+        mma_frags(bf, 4, nb, sb1, Z);
+        mma_frags(bf, 4 * ncc, nx, sb2, [&](int slot, int k) { return ZN(xnode[slot], k); });
+        t.f_xz = putf(bf.data(), bf.size() * 2);
         blob.resize((blob.size() + 15) / 16 * 16, 0);
         t.ftab_bytes = (int)(blob.size() - (size_t)t.off_ftab);
       }

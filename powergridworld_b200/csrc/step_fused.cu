@@ -15,22 +15,23 @@
 //   observations and state, and leaves real power and reward in shared memory; the agents'
 //   sums (in component order, as the reference adds them) stay on chip -- no agent_p / reward
 //   round trip through HBM, no second launch, one clock read, one staging of the event row.
-// * Power flow: warp w owns load branch w.  One iteration of u <- u0 - Zbb i(u) is: the current
-//   of my branch into a [k][env] float2 array (conflict free, double-buffered by iteration
-//   parity), one CTA barrier, then the new drop of my branch from the env's nb currents against
-//   the Zbb row (Zbb^T / xscale in shared memory, warp-uniform broadcasts), two FFMA chains on
-//   the FP32 pipe.  At 32 envs per tile a tensor-core contraction buys nothing: its latency was
-//   the hand-offs around the MMA (DESIGN.md section 4.3d).  Per-env convergence: max |d drop|
-//   over the env's 16 branch threads through a shared-memory atomicMax; converged envs freeze
-//   their currents (their drop reproduces itself); every warp knows `all envs converged` from a
-//   vote over its own lanes.
-// * Polish: the fixed point's iteration once more with correctly rounded currents, then float64
-//   sweeps u <- u0 - Zbb i(u) on the SIMT pipe, one branch per thread (the env's currents through
-//   shared memory), spread over 16 warps and -- with 32-env tiles -- over every SM of the GPU:
-//   ~0.4 us per sweep at 4096 envs instead of ~3 us in the 128-env tiles of powerflow_tc2.cu.
-// * Expansion v = w - Znb i for the nodes that are not a wye-load node: the same float32 row
-//   product against Znb^T / xscale from the fixed point's final currents, one node slot per
-//   thread and chunk of 16 slots.
+// * Power flow: the row products of u <- u0 - Zbb i(u) run on warp-level mma.sync.m16n8k16 with
+//   the split-FP16 operands of powerflow_tc2.cu (currents x xscale and Zbb x sb1 as FP16 hi + lo,
+//   hi.hi + hi.lo + lo.hi accumulated in FP32): the tile is two m-tiles of 16 envs, the realified
+//   Zbb four n-tiles of 4 branches with (Re, Im) interleaved, so warp 4m + j's D fragment holds
+//   the complex drop of branch 4j + lane % 4 for two envs -- the input of the load model, in
+//   registers.  The currents go back as FP16 hi / lo A operands (double-buffered by iteration
+//   parity, read by ldmatrix), the warps of an m-tile meet at a named barrier of their own, and
+//   each m-tile leaves the loop when its 16 envs have converged (max |d drop| per env through a
+//   shared-memory atomicMax; converged envs freeze their currents).  No tcgen05: at 32 envs a
+//   tile, its commit / mbarrier / TMEM hand-offs were the latency (DESIGN.md section 4.3d).
+// * Polish: the fixed point's iteration once more with correctly rounded currents (one more MMA
+//   product), then float64 sweeps u <- u0 - Zbb i(u) on the SIMT pipe, one branch per thread
+//   (the env's currents through shared memory), spread over 16 warps and -- with 32-env tiles --
+//   over every SM of the GPU: ~0.4 us per sweep at 4096 envs instead of ~3 us in the 128-env
+//   tiles of powerflow_tc2.cu.
+// * Expansion v = w - Znb i for the nodes that are not a wye-load node: the same MMA product
+//   against Znb x sb2 from the fixed point's final currents, n-tiles of 4 node slots.
 //
 // Compiled -fmad=false like components.cu (the component arithmetic must round like NumPy);
 // the power-flow code spells out its fused multiply-adds.
@@ -47,8 +48,15 @@ constexpr int SF_ENVS = 32;                            // envs per tile = lanes 
 constexpr int SF_WARPS = 16;
 constexpr int SF_THREADS = SF_ENVS * SF_WARPS;
 
+// The fixed point's A operands: per iteration parity and m-tile (16 envs), 16 env rows of
+// [hi: 16 branches x (Re, Im) FP16 | lo: the same | 16 bytes of padding].  The 144-byte row
+// stride puts the 8 rows of every ldmatrix phase, and the 8 env groups of every current store,
+// on distinct banks.
+constexpr int SF_AROW = 144;
+constexpr int SF_ATILE = 16 * SF_AROW;
+
 struct SfLayout {                                      // byte offsets into dynamic shared memory
-  uint32_t tab, ftab, blob, drow, irow, i32, i64, dmax, part, vn, cp, cr, act, total;
+  uint32_t tab, ftab, blob, drow, irow, ia, ld, i64, dmax, part, vn, cp, cr, act, total;
 };
 
 __host__ __device__ inline SfLayout sf_layout(const FusedParams& P) {
@@ -64,10 +72,11 @@ __host__ __device__ inline SfLayout sf_layout(const FusedParams& P) {
   L.blob = take((uint32_t)P.c.blob_bytes);
   L.drow = take((uint32_t)P.c.dstride * 8u);
   L.irow = take((uint32_t)P.c.istride * 4u + 16u);
-  L.i32 = take(2u * 16u * SF_ENVS * 8u);               // fixed-point currents, [parity][k][env] float2
+  L.ia = take(2u * 2u * SF_ATILE);                     // fixed-point A operands, [parity][m-tile]
+  L.ld = take(16u * SF_ENVS * 16u);                    // {sr, si, drop} of each branch, [k][env] float4
   L.i64 = take(16u * SF_ENVS * 16u);                   // currents of a polish sweep
-  L.dmax = take(3u * SF_ENVS * 4u);
-  L.part = take(2u * 16u * SF_ENVS * 4u);              // per-branch min / max |v| partials
+  L.dmax = take(9u * SF_ENVS * 4u);                    // convergence maxima [2][env][4] + the iterations
+  L.part = take(2u * 24u * SF_ENVS * 4u);              // min / max |v| partials: 16 warps, 8 n-tiles
   L.vn = take(16u * SF_ENVS * 8u);                     // |v| of each branch's wye node (penalty, bus voltages)
   L.cp = take((uint32_t)P.C * SF_ENVS * 8u);           // component real power
   L.cr = take((uint32_t)P.C * SF_ENVS * 8u);           // component reward
@@ -93,6 +102,63 @@ __host__ __device__ inline SfLayout sf_layout(const FusedParams& P) {
 #define SF_STAMP(k) do { } while (0)
 #endif
 
+__device__ __forceinline__ void sf_ldsm_x4(uint32_t (&r)[4], uint32_t saddr) {
+  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+               : "r"(saddr)
+               : "memory");
+}
+
+// d += a b: m16n8k16, FP16 operands, FP32 accumulators
+__device__ __forceinline__ void sf_mma(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+  asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
+      "{%0, %1, %2, %3};"
+      : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+      : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+}
+
+// The A fragments of one m-tile: 16 envs x 16 branch currents (Re, Im), hi and lo, both k-steps
+struct SfA {
+  uint32_t h0[4], l0[4], h1[4], l1[4];
+};
+
+// The shared-memory address lane `lane` hands to ldmatrix.x4 for parity 0 of m-tile m: row
+// (lane & 7) + 8 ((lane >> 3) & 1) of the 16 x 16 block, 16-byte column half lane >> 4
+__device__ __forceinline__ uint32_t sf_a_lane(const uint32_t* sIA, int m, int lane) {
+  return smem_u32(sIA) + (uint32_t)m * SF_ATILE +
+         (uint32_t)((((lane >> 3) & 1) * 8 + (lane & 7)) * SF_AROW + (lane >> 4) * 16);
+}
+
+__device__ __forceinline__ void sf_load_a(SfA& A, uint32_t a) {
+  sf_ldsm_x4(A.h0, a);
+  sf_ldsm_x4(A.l0, a + 64);
+  sf_ldsm_x4(A.h1, a + 32);
+  sf_ldsm_x4(A.l1, a + 96);
+}
+
+// The product of an m-tile's currents with n-tile (bk0, bk1) of a B image ({hi b0, hi b1, lo b0,
+// lo b1} of k-steps 0 / 1): hi.hi + hi.lo + lo.hi, the small terms first, one accumulator chain per
+// k-step.  d = {Re, Im} of output 4j + tq for env row g, then for env row g + 8.
+__device__ __forceinline__ void sf_product(float (&d)[4], const SfA& A, uint4 bk0, uint4 bk1) {
+  float d0[4] = {0.f, 0.f, 0.f, 0.f}, d1[4] = {0.f, 0.f, 0.f, 0.f};
+  sf_mma(d0, A.l0, bk0.x, bk0.y);
+  sf_mma(d1, A.l1, bk1.x, bk1.y);
+  sf_mma(d0, A.h0, bk0.z, bk0.w);
+  sf_mma(d1, A.h1, bk1.z, bk1.w);
+  sf_mma(d0, A.h0, bk0.x, bk0.y);
+  sf_mma(d1, A.h1, bk1.x, bk1.y);
+#pragma unroll
+  for (int q = 0; q < 4; ++q) d[q] = d0[q] + d1[q];
+}
+
+// A current (scaled by xscale) as its FP16 hi / lo (Re, Im) pairs into an A row, at word q of each half
+__device__ __forceinline__ void sf_put_current(uint32_t* row, int q, float2 c) {
+  const uint32_t h = t2_pack(c.x, c.y);
+  const float2 back = __half22float2(*reinterpret_cast<const __half2*>(&h));
+  row[q] = h;
+  row[16 + q] = t2_pack(c.x - back.x, c.y - back.y);
+}
+
 // IO32: the caller's actions and observations are float arrays (P.c.io32), else double.
 template <bool ANY_M5, bool IO32 = false>
 __global__ void __launch_bounds__(SF_THREADS, 1)
@@ -115,16 +181,18 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
   const Tc2Consts& kc = *reinterpret_cast<const Tc2Consts*>(sf_smem + L.ftab + t.f_kc);
   const Tc2Polish& kp = *reinterpret_cast<const Tc2Polish*>(sf_smem + L.ftab + t.f_kp);
   const int32_t* aslot = reinterpret_cast<const int32_t*>(sf_smem + L.ftab + t.f_aslot);
-  const float2* z32 = kp.z32;                          // Zbb^T / xscale
-  const float2* xz = reinterpret_cast<const float2*>(sf_smem + L.ftab + t.f_xz);   // Znb^T / xscale, [k][slot]
   unsigned char* sBlob = sf_smem + L.blob;
   double* drow = reinterpret_cast<double*>(sf_smem + L.drow);
   int32_t* irow = reinterpret_cast<int32_t*>(sf_smem + L.irow);
-  float2* sI32 = reinterpret_cast<float2*>(sf_smem + L.i32);       // [2][16][env]
+  uint32_t* sIA = reinterpret_cast<uint32_t*>(sf_smem + L.ia);     // [parity][m-tile][16 rows][36 words]
+  float4* sLd = reinterpret_cast<float4*>(sf_smem + L.ld);         // [16][env]
   double2* sI64 = reinterpret_cast<double2*>(sf_smem + L.i64);
-  int* sDmax = reinterpret_cast<int*>(sf_smem + L.dmax);           // [3][env] float bits
+  int* sDmax = reinterpret_cast<int*>(sf_smem + L.dmax);           // [parity][env][n-tile] float bits
+  int* sIters = sDmax + 2 * SF_ENVS * 4;                           // [env]: iterations, < 0 not converged
   float* sVmn = reinterpret_cast<float*>(sf_smem + L.part);        // [16][env]
   float* sVmx = sVmn + 16 * SF_ENVS;
+  float* sXmn = sVmx + 16 * SF_ENVS;                               // [8][env]: the expansion's n-tile columns
+  float* sXmx = sXmn + 8 * SF_ENVS;
   double* sVn = reinterpret_cast<double*>(sf_smem + L.vn);         // [16][env]
   double* sCp = reinterpret_cast<double*>(sf_smem + L.cp);         // [C][env]
   double* sCr = reinterpret_cast<double*>(sf_smem + L.cr);
@@ -263,24 +331,9 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
 
   const int b = w;                                     // my load branch
   const float xs = t.xscale, ds1 = t.descale1;
-  const float rds1 = 1.f / ds1;                        // a power of two: the rescaling is exact
   const float tol_s = t.tol / ds1;
   const float4 cst = t2_cst(kc, b);
   const float2 gh = ANY_M5 ? t2_gh(kc, b) : make_float2(1.f, 0.f);
-
-  // acc - sum_k z[k zs] i_k over the nb currents of my env (cur: [k][env], scaled by xscale like
-  // t2_current's; z: a column of Zbb^T or Znb^T over xscale, warp-uniform broadcasts): two FFMA
-  // chains on the FP32 pipe, summed at the end.
-  auto zdot = [&](float2 acc, const float2* z, int zs, const float2* cur) {
-    float2 a1 = make_float2(0.f, 0.f);
-#pragma unroll 2
-    for (int jj = 0; jj + 1 < pf.nb; jj += 2) {
-      t2_cmac_sub32(acc, z[jj * zs], cur[jj * SF_ENVS + lane]);
-      t2_cmac_sub32(a1, z[(jj + 1) * zs], cur[(jj + 1) * SF_ENVS + lane]);
-    }
-    if (pf.nb & 1) t2_cmac_sub32(acc, z[(pf.nb - 1) * zs], cur[(pf.nb - 1) * SF_ENVS + lane]);
-    return make_float2(acc.x + a1.x, acc.y + a1.y);
-  };
 
   uint32_t act_phase = 0;
   for (int tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
@@ -293,7 +346,6 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
     if (pf.warm_start && b < pf.nb) up = pf.u_state[(size_t)b * E + e];
     double er0 = 0.0;
     if (w < pc.A) er0 = pf.ep_ret[(size_t)w * E + e];
-    if (w < 3) sDmax[w * SF_ENVS + lane] = 0;
 
     if (first_tile) mbar_wait(&mbar_ev, 0);            // event row has landed
     if (tile_in_smem(tile)) {                          // CTA uniform
@@ -347,90 +399,158 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
 
     // ---- nominal power of my branch: base load of the event + the agents on its load
     //      (multiagent_env.py:171-181: summed per load name in agent order; opendss.py:128)
-    float sr = 0.f, si = 0.f;
+    // (the padded branches b >= nb: zero power, zero current, zero drop)
     double2 s64 = make_double2(0.0, 0.0);
-    float2 dprev = make_float2(0.f, 0.f), cur = make_float2(0.f, 0.f);
-    if (b < pf.nb) {
-      const int l = bload[b];
-      double ctl = 0.0;
-      for (int q = lptr[l]; q < lptr[l + 1]; ++q) {
-        const pgw_agent ag = agents[lidx[q]];
-        double pa = 0.0;
-        for (int ci = ag.comp_begin; ci < ag.comp_end; ++ci) pa += sCp[ci * SF_ENVS + lane];
-        ctl += pa;
+    {
+      float sr = 0.f, si = 0.f;
+      float2 dprev = make_float2(0.f, 0.f), cur = make_float2(0.f, 0.f);
+      if (b < pf.nb) {
+        const int l = bload[b];
+        double ctl = 0.0;
+        for (int q = lptr[l]; q < lptr[l + 1]; ++q) {
+          const pgw_agent ag = agents[lidx[q]];
+          double pa = 0.0;
+          for (int ci = ag.comp_begin; ci < ag.comp_end; ++ci) pa += sCp[ci * SF_ENVS + lane];
+          ctl += pa;
+        }
+        const double kw = drow[2 + l] + ctl, kvar = drow[2 + pf.nl + l];
+        const float sh = share[b] * xs;
+        sr = (float)kw * sh;
+        si = (float)kvar * sh;
+        s64 = make_double2(kw * kp.share[b], kvar * kp.share[b]);
+        dprev = make_float2(((float)up.x - cst.x) * (1.f / ds1), ((float)up.y - cst.y) * (1.f / ds1));
+        t2_current<ANY_M5>(cst, gh, dprev.x, dprev.y, ds1, sr, si, cur.x, cur.y);
       }
-      const double kw = drow[2 + l] + ctl, kvar = drow[2 + pf.nl + l];
-      const float sh = share[b] * xs;
-      sr = (float)kw * sh;
-      si = (float)kvar * sh;
-      s64 = make_double2(kw * kp.share[b], kvar * kp.share[b]);
-      dprev = make_float2(((float)up.x - cst.x) * (1.f / ds1), ((float)up.y - cst.y) * (1.f / ds1));
-      t2_current<ANY_M5>(cst, gh, dprev.x, dprev.y, ds1, sr, si, cur.x, cur.y);
-      sI32[b * SF_ENVS + lane] = cur;
+      sLd[b * SF_ENVS + lane] = make_float4(sr, si, dprev.x, dprev.y);
+      sf_put_current(sIA + (lane >> 4) * (SF_ATILE / 4) + (lane & 15) * (SF_AROW / 4), b, cur);
     }
     __syncthreads();
     SF_STAMP(6);
 
-    // ---- fixed point: iteration `it` reads the currents of parity (it - 1) & 1 and writes those
-    //      of parity it & 1 (one barrier per iteration); the convergence maxima rotate over three
-    //      slots, so that warp 0 can clear the next one before the barrier: every thread has read
-    //      it (two iterations ago) before it arrived at the previous barrier
-    int it = 0, my_it = 0;
-    bool conv = !valid, conv_ok = true;
-    while (true) {
-      ++it;
-      const int slot = it % 3;
-      if (w == 0) sDmax[((it + 1) % 3) * SF_ENVS + lane] = 0;
-      if (b < pf.nb) {
-        const float2 d = zdot(make_float2(0.f, 0.f), z32 + b, 16, sI32 + ((it - 1) & 1) * 16 * SF_ENVS);
-        const float2 dn = make_float2(d.x * rds1, d.y * rds1);
-        const float dd = fmaxf(fabsf(dn.x - dprev.x), fabsf(dn.y - dprev.y));
-        atomicMax(&sDmax[slot * SF_ENVS + lane], __float_as_int(dd));
-        if (!conv) t2_current<ANY_M5>(cst, gh, dn.x, dn.y, ds1, sr, si, cur.x, cur.y);   // converged envs keep theirs
-        sI32[((it & 1) * 16 + b) * SF_ENVS + lane] = cur;
-        dprev = dn;
-      }
-      __syncthreads();
-      if (!conv) {
-        const float d = __int_as_float(sDmax[slot * SF_ENVS + lane]);
-        conv_ok = d < tol_s;
-        conv = conv_ok || it >= pf.max_iter;
-        my_it = it;
-      }
-      if (__all_sync(0xffffffffu, conv ? 1 : 0) != 0) break;
-    }
-
-    SF_STAMP(7);
-    [[maybe_unused]] const int it_stamp = it;
-    const float2* i_fin = sI32 + (it & 1) * 16 * SF_ENVS;   // the fixed point's final currents
-    // ---- float64 polish of my branch voltage
+    // ---- fixed point on the tensor cores (mma.sync): warp 4m + j, m < 2, j < 4, computes the drops
+    //      of m-tile m (envs 16m .. 16m + 15) and n-tile j (branches 4j .. 4j + 3); thread (g, tq) =
+    //      (lane / 4, lane % 4) holds branch 4j + tq of envs 16m + g and 16m + g + 8 in its D
+    //      fragment, and runs the load model of both.  Iteration `it` reads the A operands of parity
+    //      (it - 1) & 1 and writes those of parity it & 1; the m-tile's four warps meet at a named
+    //      barrier of their own, and each m-tile leaves the loop when its 16 envs have converged.
+    //      The convergence maxima are double-buffered by parity too: a slot is written again two
+    //      iterations later, after every thread of the m-tile has read it and arrived at the barrier
+    //      in between.  Warps 8 .. 15 wait at the barrier after the loop.
     const bool polish = t.polish > 0 && pf.reward_hook;
-    double2 u64 = make_double2(kp.u0[b].x + (double)dprev.x * (double)ds1,
-                               kp.u0[b].y + (double)dprev.y * (double)ds1);
+    if (w < 8) {
+      const int m = w >> 2, j = w & 3, g = lane >> 2, tq = lane & 3;
+      const int kb = 4 * j + tq;                       // my branch
+      const bool active = kb < pf.nb;
+      const int r0 = 16 * m + g, r1 = r0 + 8;          // my env rows of the tile
+      const float4 c4 = t2_cst(kc, kb);
+      const float2 g2 = ANY_M5 ? t2_gh(kc, kb) : make_float2(1.f, 0.f);
+      const uint4* bz = reinterpret_cast<const uint4*>(sf_smem + L.ftab + t.f_xz) + (j * 32 + lane) * 2;
+      const uint4 bk0 = bz[0], bk1 = bz[1];            // k-steps 0 / 1: {hi b0, hi b1, lo b0, lo b1}
+      const float4 l0 = sLd[kb * SF_ENVS + r0], l1 = sLd[kb * SF_ENVS + r1];
+      float2 dp0 = make_float2(l0.z, l0.w), dp1 = make_float2(l1.z, l1.w);
+      float2 cu0 = make_float2(0.f, 0.f), cu1 = make_float2(0.f, 0.f);
+      if (active) {                                    // the currents of parity 0, as the writer computed them
+        t2_current<ANY_M5>(c4, g2, dp0.x, dp0.y, ds1, l0.x, l0.y, cu0.x, cu0.y);
+        t2_current<ANY_M5>(c4, g2, dp1.x, dp1.y, ds1, l1.x, l1.y, cu1.x, cu1.y);
+      }
+      bool cv0 = e_raw - lane + r0 >= P.e_hi, cv1 = e_raw - lane + r1 >= P.e_hi;   // rows past the batch
+      bool ok0 = true, ok1 = true;
+      int it0 = 0, it1 = 0;
+      const uint32_t a_lane = sf_a_lane(sIA, m, lane);
+      uint32_t* my_row0 = sIA + m * (SF_ATILE / 4) + g * (SF_AROW / 4);
+      int it = 0;
+      while (true) {
+        ++it;
+        int* dmax = sDmax + (it & 1) * SF_ENVS * 4;
+        SfA A;
+        sf_load_a(A, a_lane + (uint32_t)((it - 1) & 1) * (2 * SF_ATILE));
+        // the scaled drop: (x xscale) (Zbb x sb1) = drop / descale1
+        float d[4];
+        sf_product(d, A, bk0, bk1);
+        const float2 dn0 = make_float2(d[0], d[1]), dn1 = make_float2(d[2], d[3]);
+        // max |d drop| (float bits: non-negative floats order as ints) over the quad's 4 branches,
+        // then over the m-tile's 4 warps from [env][n-tile] after the barrier
+        int dd0 = __float_as_int(fmaxf(fabsf(dn0.x - dp0.x), fabsf(dn0.y - dp0.y)));
+        int dd1 = __float_as_int(fmaxf(fabsf(dn1.x - dp1.x), fabsf(dn1.y - dp1.y)));
+        dd0 = max(dd0, __shfl_xor_sync(0xffffffffu, dd0, 1));
+        dd1 = max(dd1, __shfl_xor_sync(0xffffffffu, dd1, 1));
+        dd0 = max(dd0, __shfl_xor_sync(0xffffffffu, dd0, 2));
+        dd1 = max(dd1, __shfl_xor_sync(0xffffffffu, dd1, 2));
+        if (tq < 2) dmax[(tq == 0 ? r0 : r1) * 4 + j] = tq == 0 ? dd0 : dd1;
+        if (active) {                                  // converged envs keep their currents
+          if (!cv0) t2_current<ANY_M5>(c4, g2, dn0.x, dn0.y, ds1, l0.x, l0.y, cu0.x, cu0.y);
+          if (!cv1) t2_current<ANY_M5>(c4, g2, dn1.x, dn1.y, ds1, l1.x, l1.y, cu1.x, cu1.y);
+        }
+        uint32_t* row = my_row0 + (it & 1) * (SF_ATILE / 2);
+        sf_put_current(row, kb, cu0);
+        sf_put_current(row + 8 * (SF_AROW / 4), kb, cu1);
+        dp0 = dn0;
+        dp1 = dn1;
+        asm volatile("bar.sync %0, 128;" ::"r"(1 + m) : "memory");
+        if (!cv0) {
+          const int4 q = reinterpret_cast<const int4*>(dmax)[r0];
+          ok0 = __int_as_float(max(max(q.x, q.y), max(q.z, q.w))) < tol_s;
+          cv0 = ok0 || it >= pf.max_iter;
+          it0 = it;
+        }
+        if (!cv1) {
+          const int4 q = reinterpret_cast<const int4*>(dmax)[r1];
+          ok1 = __int_as_float(max(max(q.x, q.y), max(q.z, q.w))) < tol_s;
+          cv1 = ok1 || it >= pf.max_iter;
+          it1 = it;
+        }
+        if (__all_sync(0xffffffffu, (cv0 && cv1) ? 1 : 0) != 0) break;
+      }
+      if (polish) {
+        // Sweep 0 of the polish, float32: the fixed point's iteration once more, from its last drop,
+        // with correctly rounded reciprocals in the currents (A operands of parity 1, free: the
+        // m-tile's last reads of it were before the loop's last barrier).  A full sweep only has
+        // to take every branch voltage from the fixed point's ~1e-7 p.u. to ~1e-8: it feeds the
+        // currents of the next sweep, whose rows the rewards read in float64, and a sweep
+        // contracts the error by more than 10x.  Its drops (p.u.) go to the hand-over below.
+        float2 c0 = make_float2(0.f, 0.f), c1 = make_float2(0.f, 0.f);
+        if (active) {
+          t2_current32<ANY_M5>(c4, g2, dp0.x, dp0.y, ds1, l0.x, l0.y, c0.x, c0.y);
+          t2_current32<ANY_M5>(c4, g2, dp1.x, dp1.y, ds1, l1.x, l1.y, c1.x, c1.y);
+        }
+        uint32_t* row = my_row0 + SF_ATILE / 2;
+        sf_put_current(row, kb, c0);
+        sf_put_current(row + 8 * (SF_AROW / 4), kb, c1);
+        asm volatile("bar.sync %0, 128;" ::"r"(1 + m) : "memory");
+        SfA A;
+        sf_load_a(A, a_lane + 2 * SF_ATILE);
+        float d[4];
+        sf_product(d, A, bk0, bk1);
+        dp0 = make_float2(d[0] * ds1, d[1] * ds1);
+        dp1 = make_float2(d[2] * ds1, d[3] * ds1);
+      }
+      // hand-over to the one-branch-per-thread phases: the last drops (scaled; p.u. after the
+      // pre-sweep), the final currents, the iterations
+      if (active) {
+        reinterpret_cast<float2*>(&sLd[kb * SF_ENVS + r0])[1] = dp0;
+        reinterpret_cast<float2*>(&sLd[kb * SF_ENVS + r1])[1] = dp1;
+      }
+      sf_put_current(my_row0, kb, cu0);                // parity 0: the expansion's A operands
+      sf_put_current(my_row0 + 8 * (SF_AROW / 4), kb, cu1);
+      if (j == 0 && tq == 0) sIters[r0] = ok0 ? it0 : -it0;
+      if (j == 0 && tq == 1) sIters[r1] = ok1 ? it1 : -it1;
+    }
+    __syncthreads();
+    SF_STAMP(7);
+#ifdef PGW_PHASE_TIMERS
+    int it_stamp = 0;                                  // the CTA's loop count: its slowest env
+    if (tid == 0)
+      for (int r = 0; r < SF_ENVS; ++r) it_stamp = max(it_stamp, abs(sIters[r]));
+#endif
+    // ---- float64 polish of my branch voltage, from the pre-sweep's drop (or the fixed point's)
+    const float4 ld = sLd[b * SF_ENVS + lane];
+    double2 u64 = polish ? make_double2(kp.u0[b].x + (double)ld.z, kp.u0[b].y + (double)ld.w)
+                         : make_double2(kp.u0[b].x + (double)ld.z * (double)ds1,
+                                        kp.u0[b].y + (double)ld.w * (double)ds1);
     const bool my_row = ((kp.rows >> b) & 1u) != 0u;
     if (polish) {
       const int sweeps = t.polish + ((kp.rows != 0u || t.polish_row >= 0) ? 1 : 0);
-      // Sweep 0 in float32: the fixed point's iteration once more, from its last drop, with
-      // correctly rounded reciprocals in the currents, into the other parity's array (free again:
-      // its last reader passed the loop's last barrier).  A full sweep only has to take every branch voltage from the fixed
-      // point's ~1e-7 p.u. to ~1e-8: it feeds the currents of the next sweep, whose rows the rewards
-      // read in float64, and a sweep contracts the error by more than 10x.  Float32 currents are
-      // half the shared-memory traffic of the float64 sweep (every thread reads all currents of
-      // its env: 14 warps x 14 x 512 B was the sweep's bound) and the FMAs run on the FP32 pipe.
-      {
-        float2* i_pre = sI32 + ((it + 1) & 1) * 16 * SF_ENVS;
-        if (b < pf.nb) {
-          float x, y;
-          t2_current32<ANY_M5>(cst, gh, dprev.x, dprev.y, ds1, sr, si, x, y);
-          i_pre[b * SF_ENVS + lane] = make_float2(x, y);
-        }
-        __syncthreads();
-        if (b < pf.nb) {
-          const float2 d = zdot(make_float2(0.f, 0.f), z32 + b, 16, i_pre);
-          u64 = make_double2(kp.u0[b].x + (double)d.x, kp.u0[b].y + (double)d.y);
-          if (t.polish == 1 && valid) pf.u_state[(size_t)b * E + e] = u64;
-        }
-      }
+      if (t.polish == 1 && valid && b < pf.nb) pf.u_state[(size_t)b * E + e] = u64;
 #pragma unroll 1
       for (int sweep = 1; sweep < sweeps; ++sweep) {
         __syncthreads();                               // everyone has read the previous currents
@@ -471,25 +591,50 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
         if (valid) pf.vmag[(size_t)n * E + e] = mag;
       }
     }
-    for (int cc = 0; cc < t.ncc; ++cc) {
-      const int slot = 16 * cc + b;                    // warp uniform
-      if (slot < t.nx) {
-        const int n = xnode[slot];
-        if (n >= 0) {
-          // - Znb i summed from zero (terms of the size of a drop), then w added once
-          const float2 dv = zdot(make_float2(0.f, 0.f), xz + slot, 16 * t.ncc, i_fin);
-          const float2 wv = wx[slot];
-          const float vr = wv.x + dv.x, vi = wv.y + dv.y;
-          const float m2 = fmaf(vr, vr, vi * vi);
-          const float mag = m2 * t2_rsqrt(fmaxf(m2, 1e-30f));
-          vmn = fminf(vmn, mag);
-          vmx = fmaxf(vmx, mag);
-          if (valid) pf.vmag[(size_t)n * E + e] = (double)mag;
-        }
-      }
-    }
     sVmn[w * SF_ENVS + lane] = vmn;
     sVmx[w * SF_ENVS + lane] = vmx;
+    // Expansion v = w - Znb i on mma.sync from the fixed point's final currents (the A operands of
+    // parity 0): warp w takes m-tile w / 8 and the n-tiles (4 slots each) w % 8, w % 8 + 8, ...;
+    // thread (g, tq) gets slot 4 nt + tq of envs 16m + g and 16m + g + 8.  - Znb i is summed from
+    // zero (terms of the size of a drop), then w is added once.
+    {
+      const int m = w >> 3, g = lane >> 2, tq = lane & 3;
+      const int r0 = 16 * m + g, r1 = r0 + 8;
+      const int e0 = e_raw - lane + r0, e1 = e0 + 8;
+      SfA A;
+      sf_load_a(A, sf_a_lane(sIA, m, lane));
+      float mn0 = 3.0e38f, mx0 = -3.0e38f, mn1 = 3.0e38f, mx1 = -3.0e38f;
+      for (int nt = w & 7; nt < 4 * t.ncc; nt += 8) {
+        const uint4* bx = reinterpret_cast<const uint4*>(sf_smem + L.ftab + t.f_xz) + ((4 + nt) * 32 + lane) * 2;
+        float d[4];                                    // - Znb i x xscale x sb2
+        sf_product(d, A, bx[0], bx[1]);
+        const int slot = 4 * nt + tq;
+        const int n = slot < t.nx ? xnode[slot] : -1;
+        if (n >= 0) {
+          const float2 wv = wx[slot];
+          const float ds2 = t.descale2;               // a power of two: exact
+          const float vr0 = wv.x + d[0] * ds2, vi0 = wv.y + d[1] * ds2;
+          const float vr1 = wv.x + d[2] * ds2, vi1 = wv.y + d[3] * ds2;
+          const float m20 = fmaf(vr0, vr0, vi0 * vi0), m21 = fmaf(vr1, vr1, vi1 * vi1);
+          const float mag0 = m20 * t2_rsqrt(fmaxf(m20, 1e-30f)), mag1 = m21 * t2_rsqrt(fmaxf(m21, 1e-30f));
+          mn0 = fminf(mn0, mag0);
+          mx0 = fmaxf(mx0, mag0);
+          mn1 = fminf(mn1, mag1);
+          mx1 = fmaxf(mx1, mag1);
+          if (e0 < P.e_hi) pf.vmag[(size_t)n * E + e0] = (double)mag0;
+          if (e1 < P.e_hi) pf.vmag[(size_t)n * E + e1] = (double)mag1;
+        }
+      }
+#pragma unroll
+      for (int s = 1; s <= 2; s <<= 1) {
+        mn0 = fminf(mn0, __shfl_xor_sync(0xffffffffu, mn0, s));
+        mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, s));
+        mn1 = fminf(mn1, __shfl_xor_sync(0xffffffffu, mn1, s));
+        mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, s));
+      }
+      if (tq == 0) { sXmn[(w & 7) * SF_ENVS + r0] = mn0; sXmx[(w & 7) * SF_ENVS + r0] = mx0; }
+      if (tq == 1) { sXmn[(w & 7) * SF_ENVS + r1] = mn1; sXmx[(w & 7) * SF_ENVS + r1] = mx1; }
+    }
     __syncthreads();                                   // magnitudes (global) and partials visible
     SF_STAMP(9);
 
@@ -522,9 +667,14 @@ __global__ void __launch_bounds__(SF_THREADS, 1)
           mn = fminf(mn, sVmn[q * SF_ENVS + lane]);
           mx = fmaxf(mx, sVmx[q * SF_ENVS + lane]);
         }
+#pragma unroll
+        for (int q = 0; q < 8; ++q) {
+          mn = fminf(mn, sXmn[q * SF_ENVS + lane]);
+          mx = fmaxf(mx, sXmx[q * SF_ENVS + lane]);
+        }
         pf.vmin[e] = (double)mn;
         pf.vmax[e] = (double)mx;
-        pf.iters[e] = conv_ok ? my_it : -my_it;
+        pf.iters[e] = sIters[lane];
         pf.viol[e] = viol;
       }
       // every agent: bus voltage, reward (minus the shared penalty), episode return
