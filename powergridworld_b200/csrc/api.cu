@@ -1314,9 +1314,13 @@ static void* device_view(pgw_env* env, const void* host) {
 
 static int enqueue_host_step(pgw_env* env, const void* actions, void* obs, double* rew,
                              uint8_t* done, bool io32, cudaStream_t s) {
-  const int E = env->E, nch = host_chunks(env, io32);
+  const int E = env->E;
+  int nch = host_chunks(env, io32);
   int bounds[pgw_env::kMaxChunks + 1];
   const int per = ((E + nch - 1) / nch + 127) / 128 * 128;          // whole 128-env tiles
+  // Whole tiles can leave the last chunks empty (600 envs in 4 chunks: 256 + 256 + 88 + 0).  An
+  // empty chunk launches nothing, so it must not count towards the clock tickets either.
+  nch = (E + per - 1) / per;
   for (int k = 0; k <= nch; ++k) bounds[k] = std::min(E, k * per);
   const unsigned int tickets = env->has_feeder ? step_pf_tickets(env, bounds, nch) : 0u;
   const size_t pitch = (size_t)E * 8, esz = io32 ? 4 : 8, io_pitch = (size_t)E * esz;
@@ -1675,8 +1679,9 @@ int pgw_debug_comp_span(pgw_env* env, long long* host_out, int ctas) {
                       (size_t)ctas * 8 * sizeof(long long), cudaMemcpyDeviceToHost));
   return PGW_OK;
 }
-int pgw_debug_num_comp_ctas(pgw_env* env) { return env ? env->num_ctas : 0; }
 #endif
+// CTAs of the component kernel's CTA table (tests check it against a mirror of the allocation)
+int pgw_debug_num_comp_ctas(pgw_env* env) { return env ? env->num_ctas : 0; }
 long long pgw_launch_count(const pgw_env* env) { return env ? env->launches : 0; }
 long long pgw_graph_captures(const pgw_env* env) { return env ? env->graph_captures : 0; }
 long long pgw_reset_count(const pgw_env* env) { return env ? env->resets : 0; }

@@ -158,6 +158,10 @@ __global__ void __launch_bounds__(64, 10) component_kernel(const CompParams p) {
       }
     }
   }
+  // A CTA whose first block lies outside [e_lo, e_hi) (a chunk of the staged host step with fewer
+  // blocks than the agent has CTAs) never entered the loop: the event-row copy may still be
+  // writing this CTA's shared memory, so it must land before the CTA exits.
+  if (first) mbar_wait(&mbar[1], 0);
   C_STAMP(6);
   if (p.pdl_trigger == 2) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   if (p.advance_clock && threadIdx.x == 0)
