@@ -15,5 +15,6 @@ mkdir -p "$BUILD"
 "$NVCC" $COMMON ${PTXAS_V:+-Xptxas -v} -c "$HERE/powerflow_tc2.cu" -o "$BUILD/powerflow_tc2.o"
 "$NVCC" $COMMON -fmad=false ${PTXAS_V:+-Xptxas -v} -c "$HERE/step_fused.cu" -o "$BUILD/step_fused.o"
 "$NVCC" $COMMON -c "$HERE/api.cu" -o "$BUILD/api.o"
-"$NVCC" -shared $ARCH -o "$OUT" "$BUILD/components.o" "$BUILD/powerflow.o" "$BUILD/powerflow_tc.o" "$BUILD/powerflow_tc2.o" "$BUILD/step_fused.o" "$BUILD/api.o" -lcudart
+"$NVCC" $COMMON -c "$HERE/tables.cpp" -o "$BUILD/tables.o"   # host only: same host flags as api.cu
+"$NVCC" -shared $ARCH -o "$OUT" "$BUILD/components.o" "$BUILD/powerflow.o" "$BUILD/powerflow_tc.o" "$BUILD/powerflow_tc2.o" "$BUILD/step_fused.o" "$BUILD/api.o" "$BUILD/tables.o" -lcudart
 echo "built $OUT"

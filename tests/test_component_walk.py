@@ -47,7 +47,7 @@ def _torch():
 
 # ------------------------------------------------------------------ the CTA table
 def walk_plan(env, budget=None):
-    """CTAs per agent: a mirror of pgw_create's water-filling allocation (api.cu)."""
+    """CTAs per agent: a mirror of build_comp_tables' water-filling allocation (tables.cpp)."""
     comps, ipar, agents = env._b.comps, env._b.ipar, list(env._agent_recs)
     A, blocks = len(agents), (env.num_envs + 63) // 64
     if budget is None:

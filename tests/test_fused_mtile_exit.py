@@ -4,6 +4,7 @@ results may depend on the 15 envs of its m-tile and on nothing else: here the ha
 need different iteration counts (one half's actions swing from one bound to the other every step,
 the other's hold still), and the same envs stepped with the halves paired differently, and in the
 other m-tile, must give the same bits.  The last tile is ragged: its second m-tile has no env."""
+import gc
 import re
 
 import numpy as np
@@ -21,6 +22,9 @@ FIELDS = (N.FIELD_VOLTAGES, N.FIELD_PF_STATE, N.FIELD_PF_ITERS, N.FIELD_EP_RETUR
 
 def _fused_kernels(env, act):
     from torch.profiler import ProfilerActivity, profile
+    # free the cyclic garbage of earlier tests (envs, profiler traces) before the session: in a long test
+    # process torch.profiler has recorded none or only some of a session's kernels without this
+    gc.collect()
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
         env.step_batch(act)
         torch.cuda.synchronize()

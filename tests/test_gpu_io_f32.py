@@ -4,6 +4,7 @@ points) on the GPU.  The kernels compute in float64 either way, so a float32 env
 ones rounded to nearest float32, bit for bit, and rewards, done flags, state, voltages, episode
 returns and power-flow state are identical.  Every kernel variant the scenarios reach is covered,
 and the kernel names torch.profiler records prove that the float32 instantiation ran."""
+import gc
 import re
 import warnings
 
@@ -50,6 +51,9 @@ def _io32_kernels(env, act):
     torch = _torch()
     from torch.profiler import ProfilerActivity, profile
     env.set_option(N.OPT_GRAPHS, 0)
+    # free the cyclic garbage of earlier tests (envs, profiler traces) before the session: in a long test
+    # process torch.profiler has recorded none or only some of a session's kernels without this
+    gc.collect()
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
         env.step_batch(act)
         torch.cuda.synchronize()

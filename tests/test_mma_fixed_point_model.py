@@ -21,7 +21,7 @@ def feeder(request, tmp_path_factory):
 
 
 def _scale_for(m):
-    """api.cu scale_for: the power of two that takes the largest entry into [8192, 16384)."""
+    """tables.cpp scale_for: the power of two that takes the largest entry into [8192, 16384)."""
     return 2.0 ** np.floor(np.log2(16384.0 / np.abs(m).max()))
 
 

@@ -94,3 +94,42 @@ def test_per_env_rosters_validate_their_inputs(tmp_path):
     from powergridworld_b200.multiagent_env import SpecBuilder
     with pytest.raises(NotImplementedError, match="256"):
         big._emit(SpecBuilder(0), 0, True)
+
+
+def _feeder(field, value):
+    def mutate(spec):
+        setattr(spec.feeder.contents, field, value)
+    return mutate
+
+
+def _branch_load(value):
+    def mutate(spec):
+        f = spec.feeder.contents
+        C.cast(f.branch_load, C.POINTER(C.c_int32 * f.nb)).contents[3] = value
+    return mutate
+
+
+def _short_event_row(spec):
+    spec.feeder.contents.nl = spec.dtab_stride // 2     # base loads: 2 + 2 nl doubles of the row
+
+
+def _staging(spec):
+    spec.itab_stride = 40 * 1024                        # event row alone: 160 kB of int32
+    for i in range(spec.num_components):
+        spec.components[i].itab_off = 0
+
+
+@pytest.mark.parametrize("make,mutate,msg", [
+    (SB.c1_env, _feeder("nb", 129), "feeder dimensions out of range (1..128 load branches)"),
+    (SB.c1_env, _branch_load(10 ** 6), "branch load index out of range"),
+    (SB.c1_env, _branch_load(-1), "branch load index out of range"),
+    (SB.c1_env, _feeder("penalty_node", 10 ** 6), "penalty node out of range"),
+    (SB.c1_env, _short_event_row, "event row too short for the feeder base loads"),
+    (SB.c1_env, _staging, "scenario tables exceed the shared-memory staging budget"),
+], ids=["nb", "branch-load-high", "branch-load-low", "penalty-node", "dtab-stride", "staging"])
+def test_feeder_and_staging_checks_come_before_the_device(make, mutate, msg):
+    """The checks of the feeder tables and of the shared-memory staging budget run on the host
+    before any CUDA call: a malformed spec is PGW_ERR_INVALID with or without a device."""
+    env = make(num_envs=4, _dry_run=True)
+    rc, got = _create(env, mutate)
+    assert (rc, got) == (INVALID, msg)

@@ -3,6 +3,7 @@
 every tc2 tile width and FP64 row count on the 123-bus-class feeders, blocks of the FP64 kernel
 that loop over several env groups, CTAs of tc2 that run several tiles (bit for bit against
 batches whose CTAs run one), and the reward-hook epilogue with four thread groups."""
+import gc
 import re
 import warnings
 
@@ -68,6 +69,9 @@ def _instantiations(torch, envs, act):
     from torch.profiler import ProfilerActivity, profile
     for e in envs:
         e.set_option(N.OPT_GRAPHS, 0)
+    # free the cyclic garbage of earlier tests (envs, profiler traces) before the session: in a long test
+    # process torch.profiler has recorded none or only some of a session's kernels without this
+    gc.collect()
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
         for e, a in zip(envs, act):
             e.step_batch(a)
